@@ -2,6 +2,7 @@
 """Benchmark of the decode hot path (BASELINE.json): decoded Mpixel/s (bit-exact).
 
     python bench.py --gpus N --steps K --warmup W [--workload NAME]      # this repository (B200)
+    python bench.py ... --dump-outputs DIR                                # + the frames of the last timed step, as .npy
     python bench.py --impl reference --gpus N --steps K --warmup W        # CPU arm: the reference's own decode_video
 
 Workloads (synthetic streams fabricated from the shipped sample, coolchic_b200.synth: the sample's latents TILED to
@@ -47,6 +48,7 @@ WORKLOADS = {
 }
 METRIC = "decoded Mpixel/s (bit-exact)"
 UNIT = "Mpixel/s"
+DUMP_LIMIT = 60 << 20  # bytes of samples written by --dump-outputs (the files stay under 64 MB with their headers)
 FP32_PEAK_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12  # CUDA-core FMA roof of a B200 at its maximum SM clock (74.5)
 
 
@@ -202,7 +204,12 @@ def main():
     ap.add_argument("--workload", default=None, choices=list(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the informational extra measurements (148 streams, batch workload at N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the frames the last timed step decoded (rank 0) to DIR/<name>.npy, "
+                         f"float32, at most {DUMP_LIMIT >> 20} MiB (a seeded sample of whole frames when they are larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -293,9 +300,9 @@ def main():
         frame_bytes = data0[8:]  # after the video header (1 intra frame)
 
         def device_step():
-            ctx.decode_many([desc], [nn_bytes], [payload], finish=[(8, wl["fmt"])])
+            outs, _ = ctx.decode_many([desc], [nn_bytes], [payload], finish=[(8, wl["fmt"])])
             t = ctx.last_timing()
-            return t["entropy_ms"], t["synthesis_ms"]
+            return t["entropy_ms"], t["synthesis_ms"], [("frame", outs[0])]
 
         def e2e_step():
             frame, _ = decode_frame(frame_bytes, reference_frames=[], device=local_rank)
@@ -313,9 +320,9 @@ def main():
         alg_bytes[0] = sum(len(j[1]) + len(j[2]) + j[0].n_symbols() for j in jobs0)
 
         def device_step():
-            ctx.decode_many([j[0] for j in jobs0], [j[1] for j in jobs0], [j[2] for j in jobs0], finish=[(8, wl["fmt"])] * len(jobs0))
+            outs, _ = ctx.decode_many([j[0] for j in jobs0], [j[1] for j in jobs0], [j[2] for j in jobs0], finish=[(8, wl["fmt"])] * len(jobs0))
             t = ctx.last_timing()
-            return t["entropy_ms"], t["synthesis_ms"]
+            return t["entropy_ms"], t["synthesis_ms"], [(f"frame{i:04d}", o) for i, o in zip(mine, outs)]
 
         def e2e_step():
             got = broadcast_byte_strings(streams, src=0, device=dev, want=mine) if world > 1 else streams
@@ -336,9 +343,10 @@ def main():
         def device_step():
             torch.cuda.synchronize()
             t0 = time.perf_counter()
-            decode_gop(data0)
+            frames = decode_gop(data0)
             torch.cuda.synchronize()
-            return (time.perf_counter() - t0) * 1e3, 0.0
+            ms = (time.perf_counter() - t0) * 1e3
+            return ms, 0.0, [(f"frame{int(k):02d}", frames[k].data) for k in sorted(frames, key=int)]
 
         def e2e_step():
             data = broadcast_byte_strings(streams, src=0, device=dev)[0] if world > 1 else streams[0]
@@ -359,7 +367,8 @@ def main():
         ev0.record()
         for _ in range(args.steps):
             flush.zero_()
-            a, b = device_step()
+            outputs = None  # release the previous step's frames before this step allocates its own
+            a, b, outputs = device_step()
             ent_ms.append(a)
             syn_ms.append(b)
         ev1.record()
@@ -376,6 +385,8 @@ def main():
             h2d, d2h = e2e_step()
         barrier()
         e2e_ms = (time.perf_counter() - t0) * 1e3 / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
     stats = torch.tensor([dev_ms, total_ms / args.steps, e2e_ms, sum(ent_ms) / args.steps], dtype=torch.float64, device=dev)
     sums = torch.tensor([float(h2d), float(d2h), float(n_sym_total[0]), float(alg_bytes[0])], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -465,6 +476,30 @@ def main():
         print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(dirname, frames):
+    """Write the decoded frames, as returned to the caller, to ``dirname/<name>.npy`` (float32; a yuv420 frame is three
+    files <name>_y / _u / _v).  When all of them exceed DUMP_LIMIT bytes, a fixed seeded sample of whole frames is written,
+    so that two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+
+    units = []
+    for name, data in frames:
+        planes = [(f"{name}_{c}", data[c]) for c in ("y", "u", "v")] if isinstance(data, dict) else [(name, data)]
+        units.append((planes, sum(4 * t.numel() for _, t in planes)))
+    keep = list(range(len(units)))
+    if sum(n for _, n in units) > DUMP_LIMIT:
+        keep, total = [], 0
+        for i in np.random.default_rng(0).permutation(len(units)):
+            if total + units[i][1] <= DUMP_LIMIT:
+                keep.append(int(i))
+                total += units[i][1]
+        keep.sort()
+    os.makedirs(dirname, exist_ok=True)
+    for i in keep:
+        for name, t in units[i][0]:
+            np.save(os.path.join(dirname, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def many_streams(ctx, synth, parse_image, n=148, distinct=24, label=None, reps=3):

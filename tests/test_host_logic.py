@@ -1,9 +1,10 @@
 """Host-side mirrors of the reference interface: headers, coding structure, writers."""
+import json
 import os
 
 import numpy as np
 import pytest
-from conftest import GOLDEN, REFERENCE, has_reference
+from conftest import GOLDEN
 
 
 def test_kodim14_headers(kodim14):
@@ -80,39 +81,29 @@ def test_coding_structure_golden():
         CodingStructure(n_frames=4, intra_pos=[0], p_pos=[2])
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not has_reference(), reason="reference checkout not present")
 def test_against_reference_classes(kodim14):
-    """In the authoring container: our host mirrors vs the reference's own classes."""
-    import sys
-
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "..", "oracle", "refshim"))
-    sys.path.insert(0, REFERENCE)
-    from coolchic.bitstream.header.header import CoolChicHeader as RefCC
-    from coolchic.utils.codingstructure import CodingStructure as RefCS
-
+    """Our host mirrors vs what the reference's own CodingStructure and CoolChicHeader computed for the same inputs
+    (tests/golden/reference_headers.json, written by oracle/gen_golden_reference_headers.py)."""
+    from coolchic_b200 import synth
     from coolchic_b200.utils.codingstructure import CodingStructure
 
-    for n, ip, pp in GOPS:
-        ours = CodingStructure(n_frames=n, intra_pos=list(ip), p_pos=list(pp))
-        ref = RefCS(n_frames=n, intra_pos=list(ip), p_pos=list(pp))
-        for i in range(n):
-            a, b = ours.get_frame_from_coding_order(i), ref.get_frame_from_coding_order(i)
-            assert (a.display_order, a.index_references, a.frame_type, a.depth) == (
-                b.display_order, b.index_references, b.frame_type, b.depth)
-    rc = RefCC()
-    rc.read_header(kodim14["data"][13:])
-    p_ref, p = rc.get_coolchic_parameter(), kodim14["header"].get_coolchic_parameter()
-    assert [tuple(s) for s in p_ref.size_per_latent] == p.size_per_latent
-    assert p_ref.input_features_ifce == p.input_features_ifce and p_ref.flag_is_hyperlatent == p.flag_is_hyperlatent
-    for hw in [(1080, 1920), (2160, 3840), (17, 33), (1, 1), (129, 7)]:
-        from coolchic_b200 import synth
-
-        h = synth.make_coolchic_header(kodim14["header"], hw, (0, 6), (4, 6))
-        r2 = RefCC()
-        r2.read_header(h.to_bytes())
-        assert [tuple(s) for s in r2.get_coolchic_parameter().size_per_latent] == h.get_coolchic_parameter().size_per_latent
-        assert r2.get_coolchic_parameter().input_features_ifce == h.get_coolchic_parameter().input_features_ifce
+    gold = json.load(open(os.path.join(GOLDEN, "reference_headers.json")))
+    assert [(g["n_frames"], g["intra_pos"], g["p_pos"]) for g in gold["coding_structures"]] == GOPS
+    for g in gold["coding_structures"]:
+        ours = CodingStructure(n_frames=g["n_frames"], intra_pos=list(g["intra_pos"]), p_pos=list(g["p_pos"]))
+        assert len(g["coding_order"]) == g["n_frames"]
+        for i, want in enumerate(g["coding_order"]):
+            a = ours.get_frame_from_coding_order(i)
+            assert [a.display_order, a.index_references, a.frame_type, a.depth] == want
+    p_ref, p = gold["kodim14"]["parameter"], kodim14["header"].get_coolchic_parameter()
+    assert [tuple(s) for s in p_ref["size_per_latent"]] == p.size_per_latent
+    assert p_ref["input_features_ifce"] == p.input_features_ifce and p_ref["flag_is_hyperlatent"] == p.flag_is_hyperlatent
+    assert [tuple(g["img_size"]) for g in gold["synthetic_headers"]] == [(1080, 1920), (2160, 3840), (17, 33), (1, 1), (129, 7)]
+    for g in gold["synthetic_headers"]:
+        h = synth.make_coolchic_header(kodim14["header"], tuple(g["img_size"]), (0, 6), (4, 6))
+        assert h.to_bytes().hex() == g["bytes"]  # the header the reference parsed
+        assert [tuple(s) for s in g["size_per_latent"]] == h.get_coolchic_parameter().size_per_latent
+        assert g["input_features_ifce"] == h.get_coolchic_parameter().input_features_ifce
 
 
 def test_exp_golomb_python(kodim14, oracle):
