@@ -27,7 +27,7 @@ ERROR_NAMES = {
 EXPORTS = [
     "ccd_version", "ccd_sizeof_desc", "ccd_last_error", "ccd_create", "ccd_destroy", "ccd_nn_count",
     "ccd_latent_count", "ccd_decode_nn", "ccd_decode_many", "ccd_decode_coolchic", "ccd_decode_latents",
-    "ccd_synthesize", "ccd_encode_latents", "ccd_finish_frame", "ccd_inter_predict", "ccd_reconstruct_frame",
+    "ccd_synthesize", "ccd_encode_latents", "ccd_encode_many", "ccd_finish_frame", "ccd_inter_predict", "ccd_reconstruct_frame",
     "ccd_pack_frame",
     "ccd_pack_samples",
     "ccd_debug_laplace_domain", "ccd_debug_last_status", "ccd_debug_launch_count", "ccd_debug_set_producer_mask", "ccd_debug_set_fused_synthesis", "ccd_last_timing",
@@ -48,6 +48,21 @@ class CcdJob(ctypes.Structure):
         ("finish_type", ctypes.c_int32),
         ("d_out_u", ctypes.c_void_p),
         ("d_out_v", ctypes.c_void_p),
+    ]
+
+
+class CcdEncodeJob(ctypes.Structure):
+    _fields_ = [
+        ("desc", ctypes.POINTER(CcdCoolChicDesc)),
+        ("nn_bytes", ctypes.c_char_p),
+        ("nn_nbytes", ctypes.c_size_t),
+        ("d_latents", ctypes.c_void_p),
+        ("d_words", ctypes.c_void_p),
+        ("cap_words", ctypes.c_int64),
+        ("d_out", ctypes.c_void_p),
+        ("n_words", ctypes.c_int64),
+        ("status", ctypes.c_int32),
+        ("slow", ctypes.c_int32),
     ]
 
 
@@ -99,6 +114,8 @@ def load_library():
         L.ccd_synthesize.argtypes = [vp, pd, vp, vp, vp, vp]
         L.ccd_encode_latents.restype = ci
         L.ccd_encode_latents.argtypes = [vp, pd, vp, ci, ctypes.c_uint64, vp, vp, i64, vp, vp, vp]
+        L.ccd_encode_many.restype = ci
+        L.ccd_encode_many.argtypes = [vp, ctypes.POINTER(CcdEncodeJob), ci, vp]
         L.ccd_finish_frame.restype = ci
         L.ccd_finish_frame.argtypes = [vp, vp, ci, ci, ci, ci, vp, vp, vp, vp]
         L.ccd_inter_predict.restype = ci
@@ -167,6 +184,7 @@ class Context:
         _check(self._lib.ccd_create(self.device, ctypes.byref(h)))
         self._h = h
         self.torch_device = torch.device("cuda", self.device)
+        self.last_slow: List[int] = []  # encode_many: symbols outside the 31-symbol window, per job
 
     def close(self) -> None:
         if getattr(self, "_h", None):
@@ -283,6 +301,63 @@ class Context:
                                             ctypes.byref(n_words), ctypes.byref(slow), self._stream()))
         payload = words[: n_words.value].cpu().numpy().astype("<u4").tobytes()
         return lat, payload, int(slow.value)
+
+    def encode_many(self, descs: Sequence[CcdCoolChicDesc], nn_bytes: Sequence[bytes], latents: Sequence,
+                    synthesize: bool = True):
+        """Range-encode n independent Cool-chics from their latents (``ccd_encode_many``): one data-parallel ARM pass
+        over all symbols of all jobs, then one range-coder warp per job.  ``latents[i]``: the job's latents in decode
+        order (coarsest grid first, each grid row-major), a tensor or array of any integer dtype with values in
+        [-64, 63].  Returns ``(payloads, outputs)``: the latent payload bytes of every job and, with ``synthesize``,
+        the raw synthesis output [1, C, H, W] of the given latents (slices of one buffer, as in ``decode_many``),
+        else None."""
+        n = len(descs)
+        dev = self.torch_device
+        lats = []
+        for i in range(n):
+            t = latents[i] if isinstance(latents[i], torch.Tensor) else torch.from_numpy(np.ascontiguousarray(latents[i]))
+            if t.numel() != descs[i].n_symbols():
+                raise ValueError(f"job {i}: {t.numel()} latents, the descriptor has {descs[i].n_symbols()} symbols")
+            if t.dtype != torch.int8 and t.numel() and (int(t.min()) < -64 or int(t.max()) > 63):
+                # checked before the int8 conversion, which would wrap such a value (int8 values are checked on the device)
+                raise ValueError(f"job {i}: latent value outside [-64, 63]")
+            lats.append(t.reshape(-1).to(dev, torch.int8).contiguous())
+        caps = [d.n_symbols() + 1 for d in descs]  # at most one word per symbol, plus the seal
+        words = torch.empty((sum(caps),), dtype=torch.int32, device=dev)
+        outs = []
+        if synthesize:
+            sizes = [d.n_out_channels * d.img_h * d.img_w for d in descs]
+            slab = torch.empty((sum(sizes),), dtype=torch.float32, device=dev)
+        jobs = (CcdEncodeJob * n)()
+        w_off, o_off = [], 0
+        off = 0
+        for i in range(n):
+            d = descs[i]
+            jobs[i].desc = ctypes.pointer(d)
+            jobs[i].nn_bytes = nn_bytes[i]
+            jobs[i].nn_nbytes = len(nn_bytes[i])
+            jobs[i].d_latents = lats[i].data_ptr()
+            jobs[i].d_words = words.data_ptr() + 4 * off
+            jobs[i].cap_words = caps[i]
+            w_off.append(off)
+            off += caps[i]
+            if synthesize:
+                out = slab[o_off:o_off + sizes[i]].view(1, d.n_out_channels, d.img_h, d.img_w)
+                jobs[i].d_out = out.data_ptr()
+                o_off += sizes[i]
+                outs.append(out)
+            else:
+                jobs[i].d_out = None
+        _check(self._lib.ccd_encode_many(self._h, jobs, n, self._stream()))
+        # the word counts are on the host now: gather the payloads on the device, then ONE copy to the host
+        counts = [int(jobs[i].n_words) for i in range(n)]
+        self.last_slow = [int(jobs[i].slow) for i in range(n)]
+        flat = torch.cat([words[w_off[i]:w_off[i] + counts[i]] for i in range(n)]) if n else words[:0]
+        host = flat.cpu().numpy().astype("<u4").tobytes()
+        payloads, at = [], 0
+        for c in counts:
+            payloads.append(host[4 * at:4 * (at + c)])
+            at += c
+        return payloads, (outs if synthesize else None)
 
     def finish_frame(self, raw: torch.Tensor, bitdepth: int, frame_data_type: str):
         """decode_frame tail: round / (420 average) / clamp / round.  raw: [1, 3, H, W] CUDA."""

@@ -1,10 +1,10 @@
 """Per-Cool-chic decode operator.
 
 Mirror of the reference's ``coolchic/bitstream/component/coolchic.py:29-207``
-(``encode_decode_coolchic(mode="decode")``): same signature, same errors, same return value
-(raw, un-clamped, un-rounded float32 synthesis output ``[1, C, H, W]``) -- but every stage
-(NN parsing, integer ARM + IFCE, range decoding, upsampling, synthesis, final resize) runs in
-``libccdec.so`` on the GPU.  ``CoolChicDecoder`` is the module-style wrapper (``load`` /
+(``encode_decode_coolchic``, both modes): same signature, same errors, same return value
+(raw, un-clamped, un-rounded float32 synthesis output ``[1, C, H, W]``, plus the Cool-chic's bytes
+in encode mode) -- but every stage (NN parsing, integer ARM + IFCE, range decoding or encoding,
+upsampling, synthesis, final resize) runs in ``libccdec.so`` on the GPU.  ``CoolChicDecoder`` is the module-style wrapper (``load`` /
 ``forward``) named in BASELINE.json; the reference itself has no such class (SURVEY F2).
 """
 from typing import List, Literal, Optional, Sequence, Tuple
@@ -26,16 +26,22 @@ def encode_decode_coolchic(
     verbosity: int = 0,
     device: int = 0,
 ) -> Tuple[Tensor, Optional[bytes]]:
-    """Decode one Cool-chic.  Returns ``(synthesis_output [1, C, H, W] float32 CUDA, None)``."""
+    """One Cool-chic through the reference operator's contract.
+
+    ``mode="decode"``: returns ``(synthesis_output [1, C, H, W] float32 CUDA, None)``.
+    ``mode="encode"``: ``enc_quantized_latent`` holds one tensor per grid in ``size_per_latent`` order (finest first,
+    hyperlatents included), each ``[1, 1, h_i, w_i]`` of any dtype.  The latents are range-coded on the device,
+    ``n_bytes_latent`` is set on ``header`` and the function returns ``(synthesis_output of those latents,
+    header.to_bytes() + bytes_nn + latent_bytes)``."""
     if mode == "encode":
-        # the encoder side of the reference operator is out of scope of the decode drop-in;
-        # the device range encoder is exposed separately (coolchic_b200.synth)
         if enc_quantized_latent is None:
             raise ValueError(
                 "Trying to encode cool_chic latent without indicating the quantized latent value. "
                 "Found enc_quantized_latent=None. It should be a list of integer Tensor."
             )
-        raise NotImplementedError("mode='encode' is not part of the decode drop-in; see coolchic_b200.synth")
+        (out, cc_bytes), = encode_coolchics([header], [bytes_nn], [enc_quantized_latent], device=device,
+                                            verbosity=verbosity)
+        return out, cc_bytes
     if mode != "decode":
         raise ValueError(f"Unknown mode {mode}")
     if dec_bytes_latent is None:
@@ -107,3 +113,52 @@ def decode_coolchics(headers: Sequence[CoolChicHeader], bytes_nn: Sequence[bytes
     descs = [desc_from_header(h) for h in headers]
     outs, _ = ctx.decode_many(descs, [bytes(b) for b in bytes_nn], [bytes(b) for b in bytes_latent], finish=finish)
     return outs
+
+
+def latents_to_decode_order(desc: CcdCoolChicDesc, latents: Sequence[Tensor]) -> Tensor:
+    """The reference encoder's per-grid latent list (``size_per_latent`` order: finest first, each ``[1, 1, h_i, w_i]``,
+    any dtype) -> the flat int8 array in decode order (coarsest grid first, each row-major) that the library codes.
+    Raises ValueError for a wrong grid count, a wrong shape or a value outside [-64, 63] (AC_MAX_VAL,
+    constants.py:9-11): the reference's range coder has no symbol for it."""
+    if len(latents) != desc.n_grids:
+        raise ValueError(f"enc_quantized_latent has {len(latents)} grids, the header describes {desc.n_grids}")
+    grids = []
+    for g in range(desc.n_grids):
+        t = latents[g]
+        if not isinstance(t, Tensor):
+            t = torch.as_tensor(t)
+        want = (1, 1, int(desc.grid_h[g]), int(desc.grid_w[g]))
+        if tuple(t.shape) != want:
+            raise ValueError(f"latent grid {g} has shape {tuple(t.shape)}, expected {want}")
+        t = t.detach().to(torch.int64)  # like the reference (FIXED_POINT_DTYPE)
+        if t.numel() and (int(t.min()) < -64 or int(t.max()) > 63):
+            raise ValueError(f"latent grid {g} holds values in [{int(t.min())}, {int(t.max())}], outside [-64, 63]")
+        grids.append(t.reshape(-1))
+    return torch.cat(grids[::-1]).to(torch.int8)
+
+
+def encode_coolchics(headers: Sequence[CoolChicHeader], bytes_nn: Sequence[bytes], latents_lists: Sequence[Sequence[Tensor]],
+                     device: int = 0, verbosity: int = 0) -> List[Tuple[Tensor, bytes]]:
+    """Encode several independent Cool-chics (all those of a GOP or of a dataset) in ONE library call: the ARM of
+    every symbol of every Cool-chic is one data-parallel pass on the GPU, then one range-coder warp per Cool-chic.
+    ``latents_lists[i]`` is Cool-chic i's ``enc_quantized_latent``.  Sets ``n_bytes_latent`` on every header and
+    returns, per Cool-chic, ``(synthesis_output [1, C, H, W], header.to_bytes() + bytes_nn + latent_bytes)``.
+    Every argument is checked before the device is touched."""
+    if not (len(headers) == len(bytes_nn) == len(latents_lists)):
+        raise ValueError("encode_coolchics: headers, bytes_nn and latents_lists differ in length")
+    descs = [desc_from_header(h) for h in headers]
+    flat = [latents_to_decode_order(d, lats) for d, lats in zip(descs, latents_lists)]
+    ctx = _native.get_context(device)
+    payloads, outs = ctx.encode_many(descs, [bytes(b) for b in bytes_nn], flat)
+    t = ctx.last_timing()
+    res = []
+    for h, nn, pay, out in zip(headers, bytes_nn, payloads, outs):
+        h.set_value("n_bytes_latent", len(pay))
+        res.append((out, h.to_bytes() + bytes(nn) + pay))
+        if verbosity:
+            print(h.pretty_string())
+        if verbosity >= 2:
+            # as in decode mode: host parse + staging + H2D | 0 (IFCE inside the ARM pass) | ARM pass + range coder |
+            # float tail
+            print(f"{t['upload_ms'] / 1e3:6.2f} {0.0:6.2f} {t['entropy_ms'] / 1e3:6.2f} {t['synthesis_ms'] / 1e3:6.2f} ")
+    return res

@@ -395,6 +395,8 @@ struct PreparedJob {
     size_t off_tailP = 0, off_tailQ = 0, off_tailRaw = 0, off_rawtmp = 0;  // inside the synthesis scratch
     // device offsets inside the upload arena
     size_t off_words = 0, off_blob = 0, off_status = 0, off_syn = 0, off_lat = 0;
+    size_t off_iv = 0;      // data-parallel encode: the symbols' intervals, inside the scratch
+    int n_tiles = 0;        // data-parallel encode: tiles of k_enc_arm
     std::vector<float> syn_f;  // dequantised synthesis weights, packed
     size_t syn_off_ot_w = 0, syn_off_ot_b = 0, syn_off_st_w = 0, syn_off_st_b = 0;
     size_t syn_off_w[CCD_MAX_SYN], syn_off_b[CCD_MAX_SYN];
@@ -988,24 +990,27 @@ int64_t ccd_decode_nn(const CcdCoolChicDesc *desc, const uint8_t *nn_bytes, size
     return decode_nn_host(desc, L, nn_bytes, nn_nbytes, out_ints);
 }
 
-// stages: bit 0 entropy, bit 1 synthesis
+// stages: bit 0 entropy, bit 1 synthesis.  mode: 0 decode, 1 / 2 the wavefront encoder (ccd_encode_latents), 3 the
+// data-parallel encoder of the latents in d_lat_in (ccd_encode_many; synthesis only for the jobs with a d_out).
+// out_caps (optional): per-job capacity of d_out_words, else out_cap for every job.
 static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int64_t *const *nn_ints, int stages,
                             const int8_t *const *d_lat_in, int mode, uint64_t seed, uint32_t *const *d_out_words,
-                            int64_t out_cap, int32_t (*statuses)[16], cudaStream_t st);
+                            int64_t out_cap, const int64_t *out_caps, int32_t (*statuses)[16], cudaStream_t st);
 
 static int decode_impl(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int64_t *const *nn_ints, int stages,
                        const int8_t *const *d_lat_in, int mode, uint64_t seed, uint32_t *const *d_out_words,
-                       int64_t out_cap, int32_t (*statuses)[16], void *cuda_stream) {
+                       int64_t out_cap, const int64_t *out_caps, int32_t (*statuses)[16], void *cuda_stream) {
     if (!ctx) return fail(CCD_ERR_ARG, "null context");
     if (n_jobs < 0 || (n_jobs > 0 && !jobs)) return fail(CCD_ERR_ARG, "bad job list");
     if (n_jobs == 0) return CCD_OK;
-    if (stages & 2)
+    if ((stages & 2) && mode != 3)
         for (int i = 0; i < n_jobs; i++)
             if (!jobs[i].d_out) return fail(CCD_ERR_ARG, "job %d: null output pointer", i);
     DeviceGuard guard(ctx->device);
     if (!guard.ok) return fail(CCD_ERR_CUDA, "cudaSetDevice(%d) failed", ctx->device);
     cudaStream_t st = (cudaStream_t)cuda_stream;
-    const int rc = decode_impl_body(ctx, jobs, n_jobs, nn_ints, stages, d_lat_in, mode, seed, d_out_words, out_cap, statuses, st);
+    const int rc =
+        decode_impl_body(ctx, jobs, n_jobs, nn_ints, stages, d_lat_in, mode, seed, d_out_words, out_cap, out_caps, statuses, st);
     if (rc != CCD_OK) {
         // every exit path leaves the context quiescent: the pinned staging buffer, the upload arena and the scratch
         // may be reused (or re-allocated) by the next call
@@ -1021,12 +1026,12 @@ static int decode_impl(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int64_t 
 
 static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int64_t *const *nn_ints, int stages,
                             const int8_t *const *d_lat_in, int mode, uint64_t seed, uint32_t *const *d_out_words,
-                            int64_t out_cap, int32_t (*statuses)[16], cudaStream_t st) {
+                            int64_t out_cap, const int64_t *out_caps, int32_t (*statuses)[16], cudaStream_t st) {
     CUDA_TRY(cudaEventRecord(ctx->ev[0], st));
 
     std::vector<PreparedJob> P((size_t)n_jobs);
-    size_t up = 0, scratch_syn = 0, scratch_lat = 0, scratch_tail = 0;
-    size_t n_tail = 0, n_tail_levels = 0;
+    size_t up = 0, scratch_syn = 0, scratch_lat = 0, scratch_tail = 0, scratch_iv = 0;
+    size_t n_tail = 0, n_tail_levels = 0, n_enc_tiles = 0;
     for (int i = 0; i < n_jobs; i++) {
         P[(size_t)i].job = &jobs[i];
         P[(size_t)i].d = jobs[i].desc;
@@ -1050,7 +1055,17 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
         up += al(64);
         J.off_syn = up;
         up += al(J.syn_f.size() * 4);
-        if (stages & 2) {
+        if (mode == 3) {
+            J.off_iv = scratch_iv;
+            scratch_iv += al((size_t)J.n_sym * 8);
+            const int chunk = J.fast ? CCD_ENC_CHUNK_FAST : CCD_ENC_CHUNK_GENERIC;
+            for (int g = 0; g < J.d->n_grids; g++) {
+                const int64_t n_chunks = (int64_t)J.d->grid_h[g] * ((J.d->grid_w[g] + chunk - 1) / chunk);
+                J.n_tiles += (int)((n_chunks + CCD_ENC_TILE_CHUNKS - 1) / CCD_ENC_TILE_CHUNKS);
+            }
+            n_enc_tiles += (size_t)J.n_tiles;
+        }
+        if ((stages & 2) && jobs[i].d_out) {
             if (jobs[i].finish_bitdepth != 0) {
                 if (jobs[i].finish_bitdepth < 1 || jobs[i].finish_bitdepth > 16 || jobs[i].finish_type < 0 || jobs[i].finish_type > 3)
                     return fail(CCD_ERR_ARG, "job %d: bad frame tail request (bitdepth %d, type %d)", i, jobs[i].finish_bitdepth, jobs[i].finish_type);
@@ -1086,13 +1101,16 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
     up += al(n_tail_levels * ccd_tail_level_job_bytes());
     const size_t off_streams = up;
     up += al(sizeof(EntStream) * (size_t)n_jobs);
+    const size_t off_enc_tiles = up;
+    up += al(sizeof(EncTile) * n_enc_tiles);
     int rc;
     if ((rc = ensure_pin(ctx, up))) return rc;
     if ((rc = ensure_dev(ctx->upload, up))) return rc;
-    if ((rc = ensure_dev(ctx->scratch, scratch_lat + al(scratch_syn) + scratch_tail + 4096))) return rc;
+    if ((rc = ensure_dev(ctx->scratch, scratch_lat + al(scratch_syn) + scratch_tail + scratch_iv + 4096))) return rc;
     unsigned char *h = ctx->h_pin, *dv = ctx->upload.p;
     unsigned char *d_scr_syn = ctx->scratch.p + scratch_lat;
     unsigned char *d_scr_tail = d_scr_syn + al(scratch_syn);
+    unsigned char *d_scr_iv = d_scr_tail + scratch_tail;
 
     // group jobs by kernel configuration so that each group is one launch
     std::vector<int> order((size_t)n_jobs);
@@ -1126,10 +1144,33 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
         S.blob = dv + J.off_blob;
         S.status = reinterpret_cast<int32_t *>(dv + J.off_status);
         S.out_words = d_out_words ? d_out_words[i] : nullptr;
-        S.out_cap = d_out_words ? out_cap : 0;
+        S.out_cap = d_out_words ? (out_caps ? out_caps[i] : out_cap) : 0;
+        if (mode == 3) {
+            S.words = reinterpret_cast<const uint32_t *>(d_scr_iv + J.off_iv);
+            S.n_words = 2 * J.n_sym;
+        }
     }
     for (int t = 0; t < n_jobs; t++)
         memcpy(h + off_streams + sizeof(EntStream) * (size_t)t, &P[(size_t)order[(size_t)t]].es, sizeof(EntStream));
+    // data-parallel encode: the tiles of k_enc_arm, launch group after launch group (stream index = position in the
+    // sorted EntStream array)
+    std::vector<size_t> enc_group_tile0;
+    if (mode == 3) {
+        EncTile *tiles = reinterpret_cast<EncTile *>(h + off_enc_tiles);
+        size_t nt = 0;
+        for (int t = 0; t < n_jobs; t++) {
+            if (t == 0 || key(order[(size_t)t]) != key(order[(size_t)t - 1])) enc_group_tile0.push_back(nt);
+            const PreparedJob &J = P[(size_t)order[(size_t)t]];
+            const int chunk = J.fast ? CCD_ENC_CHUNK_FAST : CCD_ENC_CHUNK_GENERIC;
+            for (int gi = 0; gi < J.es.n_grids; gi++) {
+                const EntGrid &Gg = J.es.grid[gi];
+                const int n_chunks = Gg.h * ((Gg.w + chunk - 1) / chunk);
+                for (int c0 = 0; c0 < n_chunks; c0 += CCD_ENC_TILE_CHUNKS)
+                    tiles[nt++] = EncTile{t, gi, c0, std::min(CCD_ENC_TILE_CHUNKS, n_chunks - c0)};
+            }
+        }
+        enc_group_tile0.push_back(nt);
+    }
 
     // ---- batched float tail: job arrays.  Launch groups: cascade level `idx` of every stream that has one
     // (planes = idx + 2), then one launch per (cinp, C) pair for the last level + synthesis (+ frame tail).
@@ -1246,7 +1287,30 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
     ctx->last_upload_bytes = up;
     CUDA_TRY(cudaEventRecord(ctx->ev[1], st));
 
-    if (stages & 1) {
+    if ((stages & 1) && mode == 3) {
+        // one data-parallel ARM pass per launch group, then the range coder of every job in one launch
+        int t = 0, g = 0;
+        while (t < n_jobs) {
+            int u = t;
+            size_t smem = 0;
+            while (u < n_jobs && key(order[(size_t)u]) == key(order[(size_t)t])) {
+                const PreparedJob &J = P[(size_t)order[(size_t)u]];
+                smem = std::max(smem, ccd_encode_smem_bytes(J.es.arm_blob_bytes, J.es.ifce_blob_max));
+                u++;
+            }
+            const PreparedJob &J0 = P[(size_t)order[(size_t)t]];
+            EntLaunchCfg cfg{J0.d->n_ctx, J0.d->flag_ifce ? J0.d->n_ifce_out : 0, J0.fast, smem, CCD_ENC_THREADS};
+            const size_t t0 = enc_group_tile0[(size_t)g], t1 = enc_group_tile0[(size_t)g + 1];
+            const int e = ccd_enc_arm_launch(reinterpret_cast<const EntStream *>(dv + off_streams),
+                                             reinterpret_cast<const EncTile *>(dv + off_enc_tiles) + t0, (int)(t1 - t0), cfg,
+                                             ctx->d_cdf, ctx->d_scale, st);
+            if (e != 0) return fail(CCD_ERR_CUDA, "encoder ARM launch failed: %s", cudaGetErrorString((cudaError_t)e));
+            t = u;
+            g++;
+        }
+        const int e = ccd_enc_range_launch(reinterpret_cast<const EntStream *>(dv + off_streams), n_jobs, st);
+        if (e != 0) return fail(CCD_ERR_CUDA, "range encoder launch failed: %s", cudaGetErrorString((cudaError_t)e));
+    } else if (stages & 1) {
         int t = 0, g = 0;
         while (t < n_jobs) {
             int u = t;
@@ -1316,7 +1380,7 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
         }
         // everything else: one stream after the other through the general kernels
         for (int i = 0; i < n_jobs; i++) {
-            if (P[(size_t)i].tail) continue;
+            if (P[(size_t)i].tail || !jobs[i].d_out) continue;
             const bool fin = jobs[i].finish_bitdepth != 0;
             float *raw_dst = fin ? reinterpret_cast<float *>(d_scr_syn + P[(size_t)i].off_rawtmp) : jobs[i].d_out;
             rc = run_synthesis(ctx, P[(size_t)i], d_lat[(size_t)i], reinterpret_cast<const float *>(dv + P[(size_t)i].off_syn),
@@ -1349,14 +1413,16 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
         memcpy(ctx->last_status, s, 64);
         if ((stages & 1) && s[0] != 0) {
             jobs[i].status = s[0];
-            if (!first) first = fail(s[0], "job %d: corrupt latent payload (range decoder desynchronised)", i);
+            if (!first)
+                first = mode == 3 ? fail(s[0], "job %d: latent value outside [-64, 63]", i)
+                                  : fail(s[0], "job %d: corrupt latent payload (range decoder desynchronised)", i);
         }
     }
     return first;
 }
 
 int ccd_decode_many(CcdContext *ctx, CcdJob *jobs, int n_jobs, void *cuda_stream) {
-    return decode_impl(ctx, jobs, n_jobs, nullptr, 3, nullptr, 0, 0, nullptr, 0, nullptr, cuda_stream);
+    return decode_impl(ctx, jobs, n_jobs, nullptr, 3, nullptr, 0, 0, nullptr, 0, nullptr, nullptr, cuda_stream);
 }
 
 int ccd_decode_coolchic(CcdContext *ctx, const CcdCoolChicDesc *desc, const uint8_t *nn_bytes, size_t nn_nbytes,
@@ -1371,7 +1437,7 @@ int ccd_decode_latents(CcdContext *ctx, const CcdCoolChicDesc *desc, const int64
     if (!d_latents || !nn_ints) return fail(CCD_ERR_ARG, "null pointer");
     CcdJob j{desc, nullptr, 0, latent_bytes, latent_nbytes, nullptr, d_latents, 0, 0, 0, nullptr, nullptr};
     const int64_t *nn[1] = {nn_ints};
-    return decode_impl(ctx, &j, 1, nn, 1, nullptr, 0, 0, nullptr, 0, nullptr, cuda_stream);
+    return decode_impl(ctx, &j, 1, nn, 1, nullptr, 0, 0, nullptr, 0, nullptr, nullptr, cuda_stream);
 }
 
 int ccd_synthesize(CcdContext *ctx, const CcdCoolChicDesc *desc, const int64_t *nn_ints, const int8_t *d_latents,
@@ -1380,7 +1446,7 @@ int ccd_synthesize(CcdContext *ctx, const CcdCoolChicDesc *desc, const int64_t *
     CcdJob j{desc, nullptr, 0, nullptr, 0, d_out, nullptr, 0, 0, 0, nullptr, nullptr};
     const int64_t *nn[1] = {nn_ints};
     const int8_t *lat[1] = {d_latents};
-    return decode_impl(ctx, &j, 1, nn, 2, lat, 0, 0, nullptr, 0, nullptr, cuda_stream);
+    return decode_impl(ctx, &j, 1, nn, 2, lat, 0, 0, nullptr, 0, nullptr, nullptr, cuda_stream);
 }
 
 int ccd_encode_latents(CcdContext *ctx, const CcdCoolChicDesc *desc, const int64_t *nn_ints, int mode, uint64_t seed,
@@ -1391,11 +1457,50 @@ int ccd_encode_latents(CcdContext *ctx, const CcdCoolChicDesc *desc, const int64
     const int64_t *nn[1] = {nn_ints};
     uint32_t *ow[1] = {d_out_words};
     int32_t stt[1][16];
-    int rc = decode_impl(ctx, &j, 1, nn, 1, nullptr, mode, seed, ow, out_cap_words, stt, cuda_stream);
+    int rc = decode_impl(ctx, &j, 1, nn, 1, nullptr, mode, seed, ow, out_cap_words, nullptr, stt, cuda_stream);
     if (rc) return rc;
     if (n_words_out) *n_words_out = stt[0][3];
     if (slow_out) *slow_out = stt[0][2];
     if (stt[0][3] > out_cap_words) return fail(CCD_ERR_ARG, "output buffer too small (%d words needed)", stt[0][3]);
+    return CCD_OK;
+}
+
+int ccd_encode_many(CcdContext *ctx, CcdEncodeJob *jobs, int n_jobs, void *cuda_stream) {
+    if (!ctx) return fail(CCD_ERR_ARG, "null context");
+    if (n_jobs < 0 || (n_jobs > 0 && !jobs)) return fail(CCD_ERR_ARG, "bad job list");
+    std::vector<CcdJob> J((size_t)n_jobs);
+    std::vector<const int8_t *> lat((size_t)n_jobs);
+    std::vector<uint32_t *> ow((size_t)n_jobs);
+    std::vector<int64_t> caps((size_t)n_jobs);
+    std::vector<int32_t> stt((size_t)n_jobs * 16, 0);
+    bool any_out = false;
+    for (int i = 0; i < n_jobs; i++) {
+        CcdEncodeJob &e = jobs[i];
+        e.n_words = 0;
+        e.status = CCD_OK;
+        e.slow = 0;
+        if (!e.d_latents || !e.d_words || e.cap_words < 1 || (!e.nn_bytes && e.nn_nbytes))
+            return fail(CCD_ERR_ARG, "job %d: null latents / output words or capacity < 1", i);
+        J[(size_t)i] = CcdJob{e.desc, e.nn_bytes, e.nn_nbytes, nullptr, 0, e.d_out, nullptr, 0, 0, 0, nullptr, nullptr};
+        lat[(size_t)i] = e.d_latents;
+        ow[(size_t)i] = e.d_words;
+        caps[(size_t)i] = e.cap_words;
+        any_out = any_out || e.d_out;
+    }
+    const int rc = decode_impl(ctx, J.data(), n_jobs, nullptr, any_out ? 3 : 1, lat.data(), 3, 0, ow.data(), 0, caps.data(),
+                               reinterpret_cast<int32_t(*)[16]>(stt.data()), cuda_stream);
+    for (int i = 0; i < n_jobs; i++) {
+        jobs[i].status = J[(size_t)i].status;
+        jobs[i].n_words = stt[(size_t)i * 16 + 3];
+        jobs[i].slow = stt[(size_t)i * 16 + 2];
+    }
+    if (rc) return rc;
+    for (int i = 0; i < n_jobs; i++)
+        if (jobs[i].n_words > jobs[i].cap_words) {
+            jobs[i].status = CCD_ERR_ARG;
+            return fail(CCD_ERR_ARG, "job %d: output buffer too small (%lld words needed, capacity %lld)", i,
+                        (long long)jobs[i].n_words, (long long)jobs[i].cap_words);
+        }
     return CCD_OK;
 }
 

@@ -44,9 +44,9 @@ struct EntStream {
     int32_t n_ctx, cf, n_hidden, has_ifce;
     int32_t ring;          // window ring entries (power of two)
     int32_t rows;          // row ring rows (power of two)
-    int32_t mode;          // 0 decode, 1 encode given latents, 2 sample + encode
+    int32_t mode;          // 0 decode, 1 encode given latents, 2 sample + encode, 3 data-parallel encode (ccd_encode.cu)
     uint32_t prod_mask;    // which of warps 0..13 produce (14 = coder helper, 15 = range coder)
-    const uint32_t *words; // compressed words (device)
+    const uint32_t *words; // compressed words (device); mode 3: the symbols' intervals, uint2 [n_symbols] in coding order
     int64_t n_words;
     int8_t *latents;       // device, decode order
     int64_t n_symbols;
@@ -90,6 +90,25 @@ bool ccd_entropy_has_fast(int n_ctx, int cf);
 int ccd_cdf_table_build(uint32_t *d_cdf, const float *d_scale, cudaStream_t st);
 int ccd_laplace_domain(const float *d_scale, int sc_lo, int sc_hi, uint32_t *d_lo, uint32_t *d_hi,
                        cudaStream_t st);
+
+// --------------------------------------------------------------------------------------
+// Data-parallel encoder of known latents (ccd_encode.cu): k_enc_arm over tiles of every job of a launch group
+// (intervals in coding order into EntStream.words), then k_enc_range, one warp per job (words into out_words,
+// status [0] error, [2] slow-path symbols, [3] words emitted).
+// --------------------------------------------------------------------------------------
+#define CCD_ENC_THREADS 256
+#define CCD_ENC_CHUNK_FAST 8       // pixels of one row per warp step: a quad of lanes per symbol
+#define CCD_ENC_CHUNK_GENERIC 32   // one lane per symbol
+#define CCD_ENC_TILE_CHUNKS 256    // chunks per CTA
+struct EncTile {
+    int32_t stream;    // index into the launch's EntStream array
+    int32_t grid;      // decode-order grid index
+    int32_t chunk0, n_chunks;
+};
+size_t ccd_encode_smem_bytes(int arm_blob_bytes, int ifce_blob_max);
+int ccd_enc_arm_launch(const EntStream *d_streams, const EncTile *d_tiles, int n_tiles, const EntLaunchCfg &cfg,
+                       const uint32_t *d_cdf, const float *d_scale, cudaStream_t st);
+int ccd_enc_range_launch(const EntStream *d_streams, int n_streams, cudaStream_t st);
 
 // --------------------------------------------------------------------------------------
 // Synthesis stage (ccd_synth.cu)

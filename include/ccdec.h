@@ -153,6 +153,36 @@ int ccd_encode_latents(CcdContext *ctx, const CcdCoolChicDesc *desc, const int64
                        uint64_t seed, int8_t *d_latents, uint32_t *d_out_words, int64_t out_cap_words,
                        int64_t *n_words_out, int32_t *slow_path_count_out, void *cuda_stream);
 
+/* One Cool-chic to ENcode from known latents.  desc / nn_bytes as in CcdJob.  d_latents: int8 latents in decode
+ * order (coarsest grid first, each grid row-major and compact, offsets as ccd_latent_count gives them), every value
+ * in [-64, 63] (AC_MAX_VAL, constants.py:9-11; anything else fails the call with CCD_ERR_ARG, nothing is clamped).
+ * d_words / cap_words: device output, little-endian u32 words of the range-coded payload; n_symbols + 1 words always
+ * suffice (a symbol renormalises at most once, plus the seal), a smaller capacity that is exceeded fails the call with
+ * CCD_ERR_ARG.  d_out (optional, may be NULL): float32 [C_out][img_h][img_w] raw synthesis output of the given
+ * latents -- what encode_decode_coolchic(mode="encode") returns as its first value.  Out: n_words, status and slow
+ * (symbols outside the 31-symbol window, coded with the exact f64 model). */
+typedef struct CcdEncodeJob {
+    const CcdCoolChicDesc *desc;
+    const uint8_t *nn_bytes;
+    size_t nn_nbytes;
+    const int8_t *d_latents;
+    uint32_t *d_words;
+    int64_t cap_words;
+    float *d_out;
+    int64_t n_words;
+    int32_t status;
+    int32_t slow;
+} CcdEncodeJob;
+
+/* Encode n independent Cool-chics: the latent half of encode_decode_coolchic(mode="encode")
+ * (component/coolchic.py:29-207, latent.py:142-173 with range_coder.encode, rangecoder.py:46-78 -> constriction
+ * RangeEncoder.encode / get_compressed) plus, for the jobs with a d_out, the same upsampling + synthesis as
+ * ccd_decode_many.  Every latent is known, so the ARM of all symbols of all jobs runs as one data-parallel pass over
+ * the GPU; only the range recursion is serial (one warp per job).  Byte-identical to ccd_encode_latents mode 1.
+ * Synchronous w.r.t. the host.  ccd_last_timing afterwards: ms[0] ARM pass + range coder, ms[1] synthesis, ms[2]
+ * host prep + H2D. */
+int ccd_encode_many(CcdContext *ctx, CcdEncodeJob *jobs, int n_jobs, void *cuda_stream);
+
 /* Tail of decode_frame for every frame type (bitstream/decode.py:191-206 with
  * io/format/yuv.py:239-256,274-300): round to the 2^b-1 grid -> (444->420 2x2 average of
  * U,V) -> clamp [0,1] -> round again.  data_type: 0 rgb, 1 yuv420, 2 yuv444.
