@@ -30,7 +30,7 @@ EXPORTS = [
     "ccd_synthesize", "ccd_encode_latents", "ccd_encode_many", "ccd_finish_frame", "ccd_inter_predict", "ccd_reconstruct_frame",
     "ccd_pack_frame",
     "ccd_pack_samples",
-    "ccd_debug_laplace_domain", "ccd_debug_last_status", "ccd_debug_launch_count", "ccd_debug_set_producer_mask", "ccd_debug_set_fused_synthesis", "ccd_last_timing",
+    "ccd_debug_laplace_domain", "ccd_debug_last_status", "ccd_debug_launch_count", "ccd_debug_set_fused_synthesis", "ccd_last_timing",
 ]
 
 
@@ -132,8 +132,6 @@ def load_library():
         L.ccd_debug_last_status.argtypes = [vp, vp]
         L.ccd_debug_launch_count.restype = ctypes.c_uint64
         L.ccd_debug_launch_count.argtypes = []
-        L.ccd_debug_set_producer_mask.restype = ci
-        L.ccd_debug_set_producer_mask.argtypes = [vp, ctypes.c_uint32]
         L.ccd_debug_set_fused_synthesis.restype = ci
         L.ccd_debug_set_fused_synthesis.argtypes = [vp, ci]
         L.ccd_last_timing.restype = ci

@@ -416,9 +416,7 @@ struct CcdContext {
     float last_ms[4] = {0, 0, 0, 0};
     int32_t last_status[16] = {0};
     uint64_t last_upload_bytes = 0;
-    uint32_t prod_mask = 0x3777u;  // warps 3, 7, 11 stay idle: the coder warp (15) owns its scheduler
     int n_sm = 148;
-    int narrow_cta = 1;  // (CCD_NARROW_CTA=0 in the environment: always 16-warp CTAs)
     int fused_synthesis = 1;       // 0: layer-by-layer kernels (ccd_debug_set_fused_synthesis, tests compare both)
     // entropy launches of different ARM architectures (e.g. intra / residue / motion streams of a GOP) run
     // side by side on these streams: each launch only fills as many SMs as it has streams
@@ -918,8 +916,6 @@ int ccd_create(int device_ordinal, CcdContext **out) {
     {
         int nsm = 0;
         if (cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device_ordinal) == cudaSuccess && nsm > 0) c->n_sm = nsm;
-        const char *env = getenv("CCD_NARROW_CTA");
-        if (env && env[0] == '0') c->narrow_cta = 0;
     }
     int rc = CCD_OK;
     do {
@@ -1136,7 +1132,7 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
         d_lat[(size_t)i] = lat;
         EntStream &S = J.es;
         S.mode = mode;
-        S.prod_mask = ctx->prod_mask;
+        S.prod_mask = CCD_PROD_MASK;
         S.seed = seed + (uint64_t)i;
         S.words = reinterpret_cast<const uint32_t *>(dv + J.off_words);
         S.n_words = (int64_t)(nbytes4 / 4);
@@ -1222,7 +1218,6 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
             if (LL.count) tail_levels.push_back(LL);
         }
         // last level + synthesis
-        const float *d_synw_base = reinterpret_cast<const float *>(dv);
         for (size_t t = 0; t < tail_order.size(); t++) {
             const int i = tail_order[t];
             PreparedJob &J = P[(size_t)i];
@@ -1230,7 +1225,6 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
             const NNLayout &L = J.L;
             const int nl = J.tail_nl, g0 = J.tail_gl[0], g1 = J.tail_gl[1];
             const float *d_synw = reinterpret_cast<const float *>(dv + J.off_syn);
-            (void)d_synw_base;
             SynLayerDev all[CCD_MAX_SYN];
             int in_ft = d->syn_in;
             for (int l = 0; l < d->n_syn_layers; l++) {
@@ -1321,8 +1315,7 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
             }
             const PreparedJob &J0 = P[(size_t)order[(size_t)t]];
             // more streams than SMs: 8-warp CTAs, two per SM (registers: 2 x 256 x 128; shared memory permitting)
-            const bool narrow = mode == 0 && ctx->narrow_cta != 0 && (u - t) > ctx->n_sm &&
-                                2 * (smem + 1024) <= (size_t)227 * 1024;
+            const bool narrow = mode == 0 && (u - t) > ctx->n_sm && 2 * (smem + 1024) <= (size_t)227 * 1024;
             EntLaunchCfg cfg{J0.d->n_ctx, J0.d->flag_ifce ? J0.d->n_ifce_out : 0, J0.fast, smem,
                              narrow ? CCD_ENT_THREADS_NARROW : CCD_ENT_THREADS};
             // group 0 on the caller's stream, the next ones on auxiliary streams forked after the upload
@@ -1368,9 +1361,7 @@ static int decode_impl_body(CcdContext *ctx, CcdJob *jobs, int n_jobs, const int
             if (h0 == d->img_h && w0 == d->img_w) continue;
             const float *raw = reinterpret_cast<const float *>(d_scr_tail + J.off_tailRaw);
             float *dst = jobs[i].d_out;
-            unsigned char *tmp = nullptr;
             if (jobs[i].finish_bitdepth != 0) return fail(CCD_ERR_UNSUPPORTED, "job %d: frame tail on a resized output", i);
-            (void)tmp;
             if (d->final_ups == 0)
                 rc = ccd_resize_nearest(raw, J.tail_C, h0, w0, dst, d->img_h, d->img_w, st);
             else
@@ -1626,12 +1617,6 @@ uint64_t ccd_debug_launch_count(void) { return g_ccd_launches; }
 int ccd_debug_set_fused_synthesis(CcdContext *ctx, int on) {
     if (!ctx) return fail(CCD_ERR_ARG, "null context");
     ctx->fused_synthesis = on ? 1 : 0;
-    return CCD_OK;
-}
-
-int ccd_debug_set_producer_mask(CcdContext *ctx, uint32_t mask) {
-    if (!ctx || (mask & 0x3fffu) == 0) return fail(CCD_ERR_ARG, "bad producer mask");
-    ctx->prod_mask = mask & 0x3fffu;
     return CCD_OK;
 }
 

@@ -113,32 +113,20 @@ __device__ __forceinline__ void sts_u32(uint32_t a, uint32_t v) {
 }
 // Flag words of the hand-offs (progress, ready, done, the meta tags) are written with release and read with acquire
 // semantics at CTA scope: what a flag announces (window / hot entries, result words, decoded symbols) is visible to
-// the thread that saw the flag.  One exception, measured (tools/ab.sh): the coder's `done` store stays a plain volatile
-// store -- a release there is a fence in front of it on the serial chain's warp; it is ordered after the coder's own
+// the thread that saw the flag.  One exception: the coder's `done` store stays a plain volatile store -- a release
+// there is a fence in front of it on the serial chain's warp (measured: +1.1 %); it is ordered after the coder's own
 // result-word stores because shared-memory stores of one warp are performed in program order, and the helper reads
-// `done` with acquire.  (-DCCD_RELEASE_DONE makes it a release store.)
+// `done` with acquire.
 __device__ __forceinline__ uint32_t lds_acq_u32(uint32_t a) {
     uint32_t v;
-#ifdef CCD_RELAXED_FLAGS
-    asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(v) : "r"(a) : "memory");
-#else
     asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(v) : "r"(a) : "memory");
-#endif
     return v;
 }
 __device__ __forceinline__ void sts_rel_u32(uint32_t a, uint32_t v) {
-#ifdef CCD_RELAXED_FLAGS
-    asm volatile("st.volatile.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory");
-#else
     asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory");
-#endif
 }
 __device__ __forceinline__ void sts_done(uint32_t a, uint32_t v) {
-#ifdef CCD_RELEASE_DONE
-    sts_rel_u32(a, v);
-#else
     asm volatile("st.volatile.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory");
-#endif
 }
 __device__ __forceinline__ void sts_u8(uint32_t a, int v) {
     asm volatile("st.volatile.shared.u8 [%0], %1;" ::"r"(a), "r"(v) : "memory");
@@ -221,9 +209,6 @@ __device__ __forceinline__ void produce_chunk(const SLoc &S, const SmemLayout &s
     need = ord_diag + (uint32_t)rel;
     PROF_T(t0);
     while ((int32_t)(lds_acq_u32(sm.ctrl) - need) < 0) {
-#ifdef CCD_SPIN_SLEEP
-        __nanosleep(CCD_SPIN_SLEEP);
-#endif
     }
     PROF_ADD(pc.wait, t0);
     PROF_T(t1);
@@ -423,10 +408,9 @@ __device__ __noinline__ void encoder_emit(const SLoc &S, Coder &c, uint32_t L0, 
 // Range DEcoder = two warps.
 //   coder  (warp 15): only the (D, R) recursion.  Its lanes enumerate SEQUENCES of the next three symbols and run
 //          the exact recursion each on its own hypothesis; one shared-memory record round trip per three symbols
-//          hands the matching lane's state to all of them (coder_grid_spec below; the design it replaced -- all
-//          lanes executing one scalar chain, blocks of four "is it the mode?" steps -- is kept behind
-//          -DCCD_CODER_BLOCKS for A/B measurements).  Measured on B200: a vote / shuffle / shared-memory round trip
-//          costs this warp 27-35 cycles, a dependent ALU op 4-5, a taken branch 10-45.
+//          hands the matching lane's state to all of them (coder_grid_spec below).  Measured on B200: a vote /
+//          shuffle / shared-memory round trip costs this warp 27-35 cycles, a dependent ALU op 4-5, a taken branch
+//          10-45.
 //   helper (warp 14): everything that is not on that recursion, 32 symbols at a time:
 //          finds how far the producers have got (contiguous valid tags -> `ready`), turns the
 //          coder's result words into symbols, writes the row ring / latent array and
@@ -441,7 +425,7 @@ struct DecState {
     uint32_t wbase;
     uint32_t slow;        // symbols decoded with the exact f64 model (outside the 31-symbol window)
     uint32_t n_far;       // symbols outside {M-1, M, M+1} (instrumented build)
-    uint32_t n_redo;      // fast groups decoded again one symbol at a time (instrumented build)
+    uint32_t n_redo;      // rounds none of whose sequences matched (instrumented build)
     int err;
 };
 
@@ -451,9 +435,8 @@ __device__ __forceinline__ uint32_t coder_word(const uint32_t *__restrict__ word
     return __ldg(words + (i < wmax ? i : wmax));
 }
 
-// The compressed words reach the coder through REGISTERS: lane l of the coder warp keeps words wbase + l and
-// wbase + 32 + l; word[wpos] is one shuffle away (requested right after a symbol, consumed by the next one: no
-// memory instruction, hence no scoreboard wait, on the serial chain).  wbase advances at group boundaries.
+// Word i of the stream, one shuffle away when lane l of the coder warp keeps words wbase + l and wbase + 32 + l
+// (the kernel reads the stream's first three words this way).
 __device__ __forceinline__ uint32_t word_at(uint32_t wcur, uint32_t wnxt, uint32_t wbase, uint32_t i) {
     const uint32_t idx = i - wbase;  // 0 .. 63
     return __shfl_sync(0xffffffffu, (idx & 32u) ? wnxt : wcur, (int)idx);
@@ -469,46 +452,16 @@ __device__ __forceinline__ uint32_t word_at(uint32_t wcur, uint32_t wnxt, uint32
 __device__ __forceinline__ uint32_t res_tag(uint32_t j) { return ((j + 1u) << 10) | 0x200u; }
 
 // ---------------------------------------------------------------------------------------------------------------
-// The scalar recursion, two tiers (cycle figures: tools/ubench/steps.cu on a B200, one warp).  TIER 2 and the far
-// path serve both coders (the symbol no sequence matched / short diagonals); the blocks of TIER 1 only the block coder.
+// The scalar recursion of one symbol, for what the speculative rounds below leave over: the symbol no sequence
+// matched, and short diagonals (cycle figures: tools/ubench/steps.cu on a B200, one warp).
 //
-// TIER 1 -- "is it the mode?", branch-free, K symbols per branch.  h = (left(M-1), left(M), left(M+1), left(M+2))
-//   of the most probable symbol M.  With scale = R >> 24, lo = scale * left(M), rn = scale * p(M), Dn = D - lo:
-//   hi32(Dn) < hi32(rn) implies both Dn < rn (the symbol is M) and rn >= 2^32 (no renormalisation); then D = Dn,
-//   R = rn and NOTHING is written.  The loop-carried chain is shift -> multiply -> R (~30 cycles / symbol for a group
-//   of four, against ~86 for a step that decides three candidates with selects and ~52 for one branch per symbol).
-//   The K flags are tested together; when one fails the state BEFORE the first failing symbol is taken from the
-//   registers of the group (selects) and that symbol goes through tier 2.
+// TIER 1 -- "is it the mode?".  h = (left(M-1), left(M), left(M+1), left(M+2)) of the most probable symbol M.  With
+//   scale = R >> 24, lo = scale * left(M), rn = scale * p(M), Dn = D - lo: hi32(Dn) < hi32(rn) implies both Dn < rn
+//   (the symbol is M) and rn >= 2^32 (no renormalisation); then D = Dn, R = rn and NOTHING is written.
 // TIER 2 -- one symbol, any case: M-1 / M / M+1 decided with selects (a branch on fresh data costs this warp ~30
-//   cycles, a select ~5), renormalisation with selects, the word from a register; anything else (`far`: ~1 % of the
-//   symbols of a natural image) searches the 32-entry window lane-parallel, then the exact f64 model.
+//   cycles, a select ~5); anything else (`far`: ~1 % of the symbols of a natural image) searches the 32-entry window
+//   lane-parallel, then the exact f64 model; then the renormalisation.
 // ---------------------------------------------------------------------------------------------------------------
-struct FastOut {
-    uint32_t t;    // window index of the decoded symbol (CCD_WIN_HALF - 1 .. CCD_WIN_HALF + 1)
-    uint32_t far;  // != 0: not one of the three candidates (everything this step produced is to be discarded)
-};
-__device__ __forceinline__ FastOut fast_step(uint64_t &D, uint64_t &R, uint32_t &w0, uint32_t &wpos, const uint32_t wcur,
-                                             const uint32_t wnxt, const uint32_t wbase, const uint4 h) {
-    const uint64_t scale = R >> 24;
-    const uint64_t P0 = scale * h.x, P1 = scale * h.y, P2 = scale * h.z, P3 = scale * h.w;
-    const bool c1 = D >= P1, c2 = D >= P2;
-    FastOut o;
-    const uint64_t nlo = c2 ? P2 : (c1 ? P1 : P0);
-    const uint64_t nhi = c2 ? P3 : (c1 ? P2 : P1);
-    const uint64_t Dn = D - nlo, Rn = nhi - nlo;
-    // none of the three candidates <=> Dn >= Rn: D < P0 wraps Dn above any Rn (Rn <= R < 2^64 - (P0 - D) would need
-    // 2^64 + D < P1), D >= P3 leaves Dn >= P3 - P2 = Rn; an empty candidate interval (left(M-1) == left(M) at the
-    // lower end of the alphabet) wraps as well
-    o.far = (uint32_t)(Dn >= Rn);
-    const bool renorm = (uint32_t)(Rn >> 32) == 0u;
-    D = renorm ? ((Dn << 32) | w0) : Dn;
-    R = renorm ? (Rn << 32) : Rn;
-    wpos += renorm ? 1u : 0u;
-    w0 = word_at(wcur, wnxt, wbase, wpos);
-    o.t = c2 ? (CCD_WIN_HALF + 1u) : (c1 ? (uint32_t)CCD_WIN_HALF : (CCD_WIN_HALF - 1u));
-    return o;
-}
-
 // Exact path of one symbol that is not M-1 / M / M+1: the whole 32-entry window at once (lane per entry:
 // one conflict-free LDS, one product, one vote -- the cost does not depend on how far from the mode the
 // symbol is), then the exact f64 model (warp-cooperative) outside the window.  Out of line, by value.
@@ -545,325 +498,14 @@ __device__ __noinline__ FarOut coder_far(uint32_t wrow, uint32_t meta_slot, cons
     return o;
 }
 
-// TIER 2 as a function: symbol j, state and word queue by value in, by value out (registers; a reference into the
-// kernel's state would put it in local memory).  A taken branch costs the coder warp ~40 cycles (instruction
-// refetch: no other warp on its scheduler hides it), so the steady loop below is straight-line code whose only
-// taken branches are this call / return and one back-edge per 2 K symbols.
+// TIER 2 as a function: symbol j, state and next word by value in, by value out (registers; a reference into the
+// kernel's state would put it in local memory).
 struct T2Out {
     uint32_t d_lo, d_hi, r_lo, r_hi, w0, wpos;
     uint32_t flags;  // 2: outside the window (exact search), 4: desynchronised, 8: far (instrumented build)
 };
-#ifdef CCD_CODER_BLOCKS
-__device__ __noinline__ T2Out coder_tier2(uint32_t res_a, uint32_t win_a, uint32_t meta_a, const float *__restrict__ scale_tab,
-                                          uint32_t ring_mask, int lane, uint32_t j, const uint4 h, uint64_t D, uint64_t R,
-                                          uint32_t w0, uint32_t wpos, const uint32_t wcur, const uint32_t wnxt,
-                                          const uint32_t wbase) {
-    const uint64_t D0 = D, R0 = R;
-    const uint32_t w00 = w0, wp0 = wpos;
-#ifdef CCD_T2_WINDOW
-    // variant: no select tree, straight to the lane-parallel window search (compact code)
-    FastOut f;
-    f.far = 1u;
-    f.t = 0u;
-    (void)h;
-#else
-    const FastOut f = fast_step(D, R, w0, wpos, wcur, wnxt, wbase, h);
-#endif
-    uint32_t rw = f.t, flags = 0u;
-    if (f.far) {
-        const uint32_t slot = j & ring_mask;
-        const uint64_t scale = R0 >> 24;
-        const FarOut o = coder_far(win_a + slot * (CCD_WIN * 4), meta_a + slot * 16u, scale_tab, lane, scale, D0);
-        uint64_t Dn = D0 - o.lo, Rn = o.hi - o.lo;
-        w0 = w00;
-        wpos = wp0;
-        if ((Rn >> 32) == 0) {
-            Dn = (Dn << 32) | w0;
-            Rn <<= 32;
-            wpos++;
-            w0 = word_at(wcur, wnxt, wbase, wpos);
-        }
-        D = Dn;
-        R = Rn;
-        rw = o.rw;
-#ifdef CCD_T2_WINDOW
-        flags = o.flags;
-#else
-        flags = o.flags | 8u;
-#endif
-    }
-    // shared-memory stores of one warp are performed in program order: this word is visible before the `done`
-    // store that follows it
-    if (rw != (uint32_t)CCD_WIN_HALF) sts_u32(res_a + (j & ring_mask) * 4u, res_tag(j) | rw);
-    T2Out r;
-    r.d_lo = (uint32_t)D;
-    r.d_hi = (uint32_t)(D >> 32);
-    r.r_lo = (uint32_t)R;
-    r.r_hi = (uint32_t)(R >> 32);
-    r.w0 = w0;
-    r.wpos = wpos;
-    r.flags = flags;
-    return r;
-}
-
-__device__ __forceinline__ void coder_grid(const SLoc &S, const SmemLayout &sm, const float *__restrict__ scale_tab,
-                                           int lane, uint32_t ord_begin, uint32_t ord_end, DecState &c,
-                                           ProfCounters &pc) {
-#ifdef CCD_ONE_BLOCK
-#define CCD_STEADY_MIN 2u
-#else
-#define CCD_STEADY_MIN 3u
-#endif
-    constexpr uint32_t K = 4;  // symbols per straight-line block
-    static_assert(K <= CCD_HOT_MIRROR, "block size");
-    const uint32_t ring_mask = (uint32_t)S.ring - 1u;
-    const uint32_t ready_a = sm.ctrl + 4u, done_a = sm.ctrl + 8u;
-    const uint32_t *__restrict__ words = S.words;
-    const uint32_t wmax = (uint32_t)S.n_words + 1u;  // words[n_words .. n_words + 3] are zero (host padding)
-    uint64_t D = c.D, R = c.R;
-    uint32_t w0 = c.w0, wpos = c.wpos, wcur = c.wcur, wnxt = c.wnxt, wbase = c.wbase;
-    uint32_t j = ord_begin;
-    uint32_t limit = ord_begin;  // symbols < limit have their window in the ring
-    uint32_t o;
-    uint4 a0, a1, a2, a3, b0, b1, b2, b3;
-    auto refresh = [&]() {
-        const uint32_t r = lds_acq_u32(ready_a);
-        limit = ((int32_t)(r - ord_end) > 0) ? ord_end : r;
-    };
-    auto advance_words = [&]() {  // the lane-held words move on (at most K words are consumed between two calls)
-        wcur = wnxt;
-        wbase += 32u;
-        wnxt = coder_word(words, wmax, wbase + 32u + (uint32_t)lane);
-    };
-    auto note_flags = [&](uint32_t fl) {  // rare: touches the (local-memory) decoder state
-        if (fl & 2u) c.slow++;
-        if (fl & 4u) c.err = CCD_ERR_DESYNC;
-#ifdef CCD_PROFILE
-        c.n_far++;
-#endif
-    };
-// tier 2 through the function (two more taken branches: used off the steady path only)
-#define CCD_TIER2(JJ, H)                                                                                              \
-    do {                                                                                                              \
-        const T2Out r_ = coder_tier2(sm.res, sm.win, sm.meta, scale_tab, ring_mask, lane, (JJ), (H), D, R, w0, wpos, wcur, \
-                                     wnxt, wbase);                                                                    \
-        D = ((uint64_t)r_.d_hi << 32) | r_.d_lo;                                                                      \
-        R = ((uint64_t)r_.r_hi << 32) | r_.r_lo;                                                                      \
-        w0 = r_.w0;                                                                                                   \
-        wpos = r_.wpos;                                                                                               \
-        if (__builtin_expect(r_.flags != 0u, 0)) note_flags(r_.flags);                                                \
-    } while (0)
-// tier 2 inline (the first failing symbol of a block): three candidates + renormalisation by selects, far by call
-#define CCD_T2_INLINE(JJ, H)                                                                                          \
-    {                                                                                                                 \
-        const uint64_t D0_ = D, R0_ = R;                                                                              \
-        const uint32_t w00_ = w0, wp0_ = wpos;                                                                        \
-        const FastOut f_ = fast_step(D, R, w0, wpos, wcur, wnxt, wbase, (H));                                         \
-        uint32_t rw_ = f_.t;                                                                                          \
-        if (__builtin_expect(f_.far != 0u, 0)) {                                                                      \
-            const uint32_t slot_ = (JJ) & ring_mask;                                                                  \
-            const FarOut o_ = coder_far(sm.win + slot_ * (CCD_WIN * 4), sm.meta + slot_ * 16u, scale_tab, lane, R0_ >> 24, D0_); \
-            uint64_t Dn_ = D0_ - o_.lo, Rn_ = o_.hi - o_.lo;                                                          \
-            w0 = w00_;                                                                                                \
-            wpos = wp0_;                                                                                              \
-            if ((Rn_ >> 32) == 0) {                                                                                   \
-                Dn_ = (Dn_ << 32) | w0;                                                                               \
-                Rn_ <<= 32;                                                                                           \
-                wpos++;                                                                                               \
-                w0 = word_at(wcur, wnxt, wbase, wpos);                                                                \
-            }                                                                                                         \
-            D = Dn_;                                                                                                  \
-            R = Rn_;                                                                                                  \
-            rw_ = o_.rw;                                                                                              \
-            note_flags(o_.flags | 8u);                                                                                \
-        }                                                                                                             \
-        if (rw_ != (uint32_t)CCD_WIN_HALF) sts_u32(sm.res + ((JJ) & ring_mask) * 4u, res_tag(JJ) | rw_);              \
-    }
-// K tier-1 steps on entries H0..H3; bad_i != 0 when symbol i is not "the mode, no renormalisation"
-#define CCD_BLOCK(H0, H1, H2, H3)                                                                                     \
-    uint64_t Ds1, Rs1, Ds2, Rs2, Ds3, Rs3, Ds4, Rs4;                                                                  \
-    uint32_t bad0, bad1, bad2, bad3;                                                                                  \
-    {                                                                                                                 \
-        uint64_t sc_ = R >> 24;                                                                                       \
-        Rs1 = sc_ * ((H0).z - (H0).y);                                                                                \
-        Ds1 = D - sc_ * (H0).y;                                                                                       \
-        bad0 = (uint32_t)(Ds1 >> 32) >= (uint32_t)(Rs1 >> 32);                                                        \
-        sc_ = Rs1 >> 24;                                                                                              \
-        Rs2 = sc_ * ((H1).z - (H1).y);                                                                                \
-        Ds2 = Ds1 - sc_ * (H1).y;                                                                                     \
-        bad1 = (uint32_t)(Ds2 >> 32) >= (uint32_t)(Rs2 >> 32);                                                        \
-        sc_ = Rs2 >> 24;                                                                                              \
-        Rs3 = sc_ * ((H2).z - (H2).y);                                                                                \
-        Ds3 = Ds2 - sc_ * (H2).y;                                                                                     \
-        bad2 = (uint32_t)(Ds3 >> 32) >= (uint32_t)(Rs3 >> 32);                                                        \
-        sc_ = Rs3 >> 24;                                                                                              \
-        Rs4 = sc_ * ((H3).z - (H3).y);                                                                                \
-        Ds4 = Ds3 - sc_ * (H3).y;                                                                                     \
-        bad3 = (uint32_t)(Ds4 >> 32) >= (uint32_t)(Rs4 >> 32);                                                        \
-    }
-// first failing symbol f of the block: state before it by selects, the hot entries of the K symbols after it are
-// requested (their latency hides behind tier 2), tier 2 through the function, back to the top
-#define CCD_RECOVER(H0, H1, H2, H3)                                                                                   \
-    {                                                                                                                 \
-        uint32_t f_ = 3u;                                                                                             \
-        uint4 hf_ = (H3);                                                                                             \
-        uint64_t Df_ = Ds3, Rf_ = Rs3;                                                                                \
-        if (bad2) { f_ = 2u; hf_ = (H2); Df_ = Ds2; Rf_ = Rs2; }                                                      \
-        if (bad1) { f_ = 1u; hf_ = (H1); Df_ = Ds1; Rf_ = Rs1; }                                                      \
-        if (bad0) { f_ = 0u; hf_ = (H0); Df_ = D; Rf_ = R; }                                                          \
-        D = Df_;                                                                                                      \
-        R = Rf_;                                                                                                      \
-        j += f_;                                                                                                      \
-        o = sm.hot + ((j + 1u) & ring_mask) * 16u;                                                                    \
-        a0 = lds_v4(o);                                                                                               \
-        a1 = lds_v4(o + 16u);                                                                                         \
-        a2 = lds_v4(o + 32u);                                                                                         \
-        a3 = lds_v4(o + 48u);                                                                                         \
-        CCD_T2_INLINE(j, hf_)                                                                                         \
-        j++;                                                                                                          \
-        sts_done(done_a, j);                                                                                           \
-        PROF_COUNT_RECOVER(f_);                                                                                       \
-    }
-#ifdef CCD_PROFILE
-#define PROF_COUNT_RECOVER(F) do { pc.seg[3] += (F); c.n_redo++; } while (0)
-#else
-#define PROF_COUNT_RECOVER(F)
-#endif
-    while (j != ord_end) {
-        if ((int32_t)(limit - j) <= 0) {
-            PROF_T(t0);
-            do {
-                refresh();
-            } while ((int32_t)(limit - j) <= 0);
-            PROF_ADD(pc.wait, t0);
-        }
-        if (wpos - wbase >= 32u) advance_words();
-        if ((int32_t)(limit - j) < (int32_t)(CCD_STEADY_MIN * K) && (int32_t)(limit - j) >= (int32_t)K) {
-            // fewer symbols ready than the steady loop wants (short diagonals): one block, entries requested now
-            o = sm.hot + (j & ring_mask) * 16u;
-            a0 = lds_v4(o);
-            a1 = lds_v4(o + 16u);
-            a2 = lds_v4(o + 32u);
-            a3 = lds_v4(o + 48u);
-            CCD_BLOCK(a0, a1, a2, a3)
-            if ((bad0 | bad1 | bad2 | bad3) != 0u) {
-                CCD_RECOVER(a0, a1, a2, a3)
-            } else {
-                D = Ds4;
-                R = Rs4;
-                j += K;
-                sts_done(done_a, j);
-#ifdef CCD_PROFILE
-                pc.seg[3] += K;
-#endif
-            }
-            continue;
-        }
-        if ((int32_t)(limit - j) < (int32_t)(CCD_STEADY_MIN * K)) {
-            // the coder is close behind the producers (small grids, where the ARM latency bounds the stream);
-            // (same bound as the steady loop's: between the two nothing would be decoded)
-            const uint4 hh = lds_v4(sm.hot + (j & ring_mask) * 16u);
-            {
-                const uint64_t scale_ = R >> 24;
-                const uint64_t lo_ = scale_ * hh.y, rn_ = scale_ * (hh.z - hh.y);
-                const uint64_t dn_ = D - lo_;
-                if ((uint32_t)(dn_ >> 32) < (uint32_t)(rn_ >> 32)) {  // tier 1
-                    D = dn_;
-                    R = rn_;
-                } else {
-                    CCD_TIER2(j, hh);
-                }
-            }
-            j++;
-            sts_done(done_a, j);
-#ifdef CCD_PROFILE
-            pc.seg[4]++;
-#endif
-            continue;
-        }
-        // ---- steady state: blocks of K symbols, branch-free (tier 1 on every symbol, flags and intermediate states
-        // kept in registers), ONE branch per block; two blocks per iteration with the roles of the two sets of hot
-        // entries swapped (no copies).  A far taken branch costs this warp ~40 cycles (instruction refetch; nothing
-        // else runs on its scheduler), a short forward skip ~11.
-        o = sm.hot + (j & ring_mask) * 16u;  // (the ring's first entries are mirrored behind its end)
-        a0 = lds_v4(o);
-        a1 = lds_v4(o + 16u);
-        a2 = lds_v4(o + 32u);
-        a3 = lds_v4(o + 48u);
-        while (true) {
-            // (K entries in a0..a3 valid for j; 2 K more must be ready for the two prefetches of this iteration)
-            // (the two rare maintenance cases behind ONE test: every skipped block is a taken branch for this warp)
-            if (((int32_t)(limit - j) < (int32_t)(CCD_STEADY_MIN * K)) | (wpos - wbase >= 32u)) {
-                if (wpos - wbase >= 32u) advance_words();
-                if ((int32_t)(limit - j) < (int32_t)(CCD_STEADY_MIN * K)) {
-                    refresh();
-                    if ((int32_t)(limit - j) < (int32_t)(CCD_STEADY_MIN * K)) break;
-                }
-            }
-            o = sm.hot + ((j + K) & ring_mask) * 16u;
-            b0 = lds_v4(o);
-            b1 = lds_v4(o + 16u);
-            b2 = lds_v4(o + 32u);
-            b3 = lds_v4(o + 48u);
-            {
-                CCD_BLOCK(a0, a1, a2, a3)
-                if ((bad0 | bad1 | bad2 | bad3) != 0u) {
-                    CCD_RECOVER(a0, a1, a2, a3)
-                    continue;
-                }
-                D = Ds4;
-                R = Rs4;
-            }
-#ifdef CCD_ONE_BLOCK
-            // variant: one block per iteration (the steady loop needs 2 K ready symbols instead of 3 K), entries copied
-            j += K;
-            sts_done(done_a, j);
-            a0 = b0;
-            a1 = b1;
-            a2 = b2;
-            a3 = b3;
-            continue;
-#endif
-            sts_done(done_a, j + K);  // every lane stores the same word: no predicate on the hot path
-            o = sm.hot + ((j + 2u * K) & ring_mask) * 16u;
-            a0 = lds_v4(o);
-            a1 = lds_v4(o + 16u);
-            a2 = lds_v4(o + 32u);
-            a3 = lds_v4(o + 48u);
-            {
-                CCD_BLOCK(b0, b1, b2, b3)
-                if ((bad0 | bad1 | bad2 | bad3) != 0u) {
-                    j += K;
-                    CCD_RECOVER(b0, b1, b2, b3)
-                    continue;
-                }
-                D = Ds4;
-                R = Rs4;
-            }
-            j += 2u * K;
-            sts_done(done_a, j);
-#ifdef CCD_PROFILE
-            pc.seg[3] += 2 * K;
-#endif
-        }
-    }
-#undef CCD_BLOCK
-#undef CCD_RECOVER
-#undef CCD_T2_INLINE
-#undef CCD_TIER2
-    c.D = D;
-    c.R = R;
-    c.w0 = w0;
-    c.wpos = wpos;
-    c.wcur = wcur;
-    c.wnxt = wnxt;
-    c.wbase = wbase;
-}
-
-#endif  // CCD_CODER_BLOCKS
-
 // ---------------------------------------------------------------------------------------------------------------
-// SPECULATIVE coder (default): the lanes of the coder warp enumerate SYMBOL SEQUENCES.
+// SPECULATIVE coder: the lanes of the coder warp enumerate SYMBOL SEQUENCES.
 //   Lane l = c1 + 3 c2 + 9 c3 (27 lanes) assumes that the next three symbols are M1-1+c1, M2-1+c2, M3-1+c3 (Mi = the
 //   most probable symbol of symbol i) and runs the exact recursion -- interval test, update, renormalisation by
 //   selects -- on its OWN copy of (D, R): no branch, no vote, no shuffle inside the three steps (a vote / shuffle /
@@ -898,7 +540,7 @@ __device__ __forceinline__ uint2 lds_v2(uint32_t a) {
     return v;
 }
 
-// TIER 2 of the speculative coder (one symbol, any case; out of line, rare): as coder_tier2, the words from memory.
+// TIER 2: one symbol, any case (out of line, rare).  After a renormalisation the next word is read from memory.
 __device__ __noinline__ T2Out coder_tier2_g(uint32_t res_a, uint32_t win_a, uint32_t meta_a, const float *__restrict__ scale_tab,
                                             uint32_t ring_mask, int lane, uint32_t j, const uint4 h, uint64_t D, uint64_t R,
                                             uint32_t w0, uint32_t wpos, const uint32_t *__restrict__ words, uint32_t wmax) {
@@ -907,9 +549,12 @@ __device__ __noinline__ T2Out coder_tier2_g(uint32_t res_a, uint32_t win_a, uint
     const bool c1 = D >= P1, c2 = D >= P2;
     const uint64_t nlo = c2 ? P2 : (c1 ? P1 : P0);
     const uint64_t nhi = c2 ? P3 : (c1 ? P2 : P1);
-    uint64_t Dn = D - nlo, Rn = nhi - nlo;  // (none of the three <=> Dn >= Rn: see fast_step)
+    uint64_t Dn = D - nlo, Rn = nhi - nlo;
     uint32_t rw = c2 ? (CCD_WIN_HALF + 1u) : (c1 ? (uint32_t)CCD_WIN_HALF : (CCD_WIN_HALF - 1u));
     uint32_t flags = 0u;
+    // none of the three candidates <=> Dn >= Rn: D < P0 wraps Dn above any Rn (Rn <= R < 2^64 - (P0 - D) would need
+    // 2^64 + D < P1), D >= P3 leaves Dn >= P3 - P2 = Rn; an empty candidate interval (left(M-1) == left(M) at the
+    // lower end of the alphabet) wraps as well
     if (Dn >= Rn) {
         const uint32_t slot = j & ring_mask;
         const FarOut o = coder_far(win_a + slot * (CCD_WIN * 4), meta_a + slot * 16u, scale_tab, lane, scale, D);
@@ -1041,11 +686,6 @@ __device__ __forceinline__ void coder_grid_spec(const SLoc &S, const SmemLayout 
     }
 // one round on set X; failed != 0 afterwards when no sequence matched (state advanced over the decided prefix)
 // (shared-memory accesses of one warp are performed in program order: the record is read back without a barrier)
-#ifdef CCD_SPEC_SYNCWARP
-#define CCD_SPEC_SYNC() __syncwarp()
-#else
-#define CCD_SPEC_SYNC()
-#endif
 #define CCD_RSTEPS(X)                                                                                                 \
         uint32_t dl = (uint32_t)D, dh = (uint32_t)(D >> 32), rl = (uint32_t)R, rh = (uint32_t)(R >> 32);              \
         uint32_t ok = live, k = 0u;                                                                                   \
@@ -1061,7 +701,6 @@ __device__ __forceinline__ void coder_grid_spec(const SLoc &S, const SmemLayout 
         sts_u32_if(ok & ner, sm.res + ((j & ring_mask) << 2), (j << 10) + CR);                                        \
         sts_v4_if(ok, rec_a, dl, dh, rl, rh);                                                                         \
         sts_v2_if(ok, rec_a + 16u, k, tag_);                                                                          \
-        CCD_SPEC_SYNC();                                                                                              \
         const uint4 rv_ = lds_v4(rec_a);                                                                              \
         const uint2 rt_ = lds_v2(rec_a + 16u);
 // (the three macros share the names the steps define)
@@ -1335,7 +974,7 @@ __global__ void __launch_bounds__(CCD_ENT_THREADS, 1)
     const EntStream &G = streams[blockIdx.x];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     // role assignment: the last warp = range coder (recursion), the one before = its helper; producer warps are those
-    // enabled in prod_mask (by default the coder keeps its scheduler partition for itself: warps 3, 7, 11 idle).  The
+    // enabled in prod_mask (CCD_PROD_MASK: the coder keeps its scheduler partition for itself, warps 3, 7, 11 idle).  The
     // CTA has 16 warps, or 8 when the call holds more streams than the GPU has SMs (two CTAs per SM then: the two coder
     // warps share the scheduler the idle warps leave to them, each issuing ~40 % of the time)
     const int nw = (int)(blockDim.x >> 5);
@@ -1417,11 +1056,7 @@ __global__ void __launch_bounds__(CCD_ENT_THREADS, 1)
         const uint32_t n_sym = (uint32_t)sm.grid->h * (uint32_t)sm.grid->w;
         PROF_T(tg);
         if (is_coder) {
-#ifdef CCD_CODER_BLOCKS
-            if (S.mode == 0) coder_grid(S, sm, scale_tab, lane, ord, ord + n_sym, ds, pc);
-#else
             if (S.mode == 0) coder_grid_spec(S, sm, scale_tab, lane, ord, ord + n_sym, ds, pc);
-#endif
             else if (S.mode == 1) encode_grid<1>(S, sm, scale_tab, lane, ord, ord + n_sym, cd);
             else encode_grid<2>(S, sm, scale_tab, lane, ord, ord + n_sym, cd);
         } else if (is_helper) {
@@ -1435,8 +1070,8 @@ __global__ void __launch_bounds__(CCD_ENT_THREADS, 1)
 #ifdef CCD_PROFILE
     // status words of the instrumented build (kilo-cycles unless stated): [4] coder wait, [5] coder total,
     // [6..9] producers (summed over the warps): wait, ARM, window fetch + publication, total, [10] symbols outside
-    // {M-1, M, M+1}, [11] fast groups decoded again, [12] symbols decoded one at a time, [13] symbols decoded in
-    // fast groups, [14] chunks produced, [15] helper total
+    // {M-1, M, M+1}, [11] rounds none of whose sequences matched, [12] symbols decoded one at a time, [13] symbols
+    // decided in rounds, [14] chunks produced, [15] helper total
     if (lane == 0) {
         if (is_helper) {
             G.status[15] = (int)(pc.total >> 10);

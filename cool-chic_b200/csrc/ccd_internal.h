@@ -13,6 +13,7 @@
 #define CCD_ENT_THREADS_NARROW 256   // 5 producer warps + helper + coder: two streams per SM when a call holds more streams than SMs
 #define CCD_ENT_WARPS (CCD_ENT_THREADS / 32)
 #define CCD_ENT_PRODUCERS (CCD_ENT_WARPS - 2)
+#define CCD_PROD_MASK 0x3777u        // producer warps: 3, 7, 11 stay idle, so the coder warp (15) owns its scheduler
 #define CCD_WIN 32                   // cumulative-window entries per symbol (31 decodable symbols)
 #define CCD_WIN_HALF 14              // window = symbols mu_int-14 .. mu_int+16; the mode sits at the EVEN index 14
                                      // so that (left(mode), left(mode+1)) is one aligned LDS.64

@@ -436,7 +436,7 @@ __global__ void __launch_bounds__(SF_THREADS) k_syn_fused(SynFusedParams P) {
 //
 //   k_ups_level_b : one level of the cascade for ALL streams of a group in one launch
 //                   (blockIdx.z = stream * planes + plane)
-//   k_tail_syn    : the LAST cascade level + the whole synthesis + the frame tail in one kernel.  The dense
+//   k_tail_syn2   : the LAST cascade level + the whole synthesis + the frame tail in one kernel.  The dense
 //                   latent at image resolution (7 fp32 planes, 28 B / pixel written and read back by the
 //                   unfused path) is never materialised: a CTA stages the int8 tile of the finest grid
 //                   (zero padding = TMA out-of-bounds fill) and the tile of the half-resolution stack in shared
@@ -545,346 +545,9 @@ __host__ __device__ inline int ts_sh(int n3) { return (SF_TH + 2 * n3) / 2 + 5; 
 __device__ __forceinline__ float quant(float v, float M);
 __device__ __forceinline__ float clamp01(float v);
 
-template <int CINP, int C>
-__global__ void __launch_bounds__(SF_THREADS) k_tail_syn(const TailSynJob *__restrict__ jobs) {
-    extern __shared__ __align__(128) unsigned char ts_raw[];
-    const TailSynJob &P = jobs[blockIdx.z];
-    const int H = P.h, W = P.w;
-    const int x0 = blockIdx.x * SF_TW, y0 = blockIdx.y * SF_TH;
-    if (x0 >= W || y0 >= H) return;  // (streams of one launch may have different sizes)
-    const int n3 = P.n3, hid = P.hid, cin = P.cin, cc = cin - 1;
-    const int RW = SF_TW + 2 * n3, RH = SF_TH + 2 * n3;  // stage-A region
-    const int LW = ts_lw(n3), LH = ts_lh(n3), SW = ts_sw(n3), SH = ts_sh(n3);
-    constexpr int CP = (C + 3) & ~3;
-    // shared memory: [mbarrier 16 B] [latent tile] [stack tile] | weights, region buffers (floats)
-    uint64_t *bar = reinterpret_cast<uint64_t *>(ts_raw);
-    int8_t *Lt = reinterpret_cast<int8_t *>(ts_raw + 128);                          // [LH][LW]
-    float *St = reinterpret_cast<float *>(ts_raw + 128 + ((LW * LH + 127) & ~127)); // [cc][SH][SW]
-    float *sw0 = St + ((cc * SH * SW + 31) & ~31);  // [hid][CINP]
-    float *sb0 = sw0 + hid * CINP;
-    float *sw1 = sb0 + hid;                  // [hid][CP]
-    float *sb1 = sw1 + hid * CP;
-    float *sw3 = sb1 + CP;                   // [2][C][C][9]
-    float *sb3 = sw3 + 2 * C * C * 9;
-    float *sws = sb3 + 2 * CP;               // [C][CINP]
-    float *sbs = sws + C * CINP;
-    float *swo = sbs + CP;                   // [C][CP]
-    float *sbo = swo + C * CP;
-    float *skt = sbo + CP;                   // [8][8]
-    float *skc = skt + 64;                   // [7][7] (+ pad)
-    float *bufA = skc + 52;                  // [C][RH][RW]
-    float *bufB = bufA + C * RH * RW;        // [C][RH-2][RW-2]   (n3 == 2)
-    float *sstab = bufB + (n3 == 2 ? C * (RH - 2) * (RW - 2) : 0);  // [C][SF_TH][SF_TW]
-    const int tid = threadIdx.x;
-    // tile origins (frame coordinates of element 0 of the tiles)
-    const int Y0 = y0 - n3, X0 = x0 - n3;                   // stage-A region
-    const int ly0 = Y0 - 3, lx0 = (X0 - 3) & ~15;           // latent tile (16-byte aligned start)
-    const int sy0 = ((Y0 < 0 ? 0 : Y0) >> 1) - 2, sx0 = (((X0 < 0 ? 0 : X0) >> 1) - 2) & ~3;  // stack tile
-    const int ch = P.ch, cw = P.cw;
-    // ---- stage 0: tiles -> shared memory
-    if (P.use_tma) {
-        const uint32_t bar_a = (uint32_t)__cvta_generic_to_shared(bar);
-        if (tid == 0) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        __syncthreads();
-        if (tid == 0) {
-            const uint32_t bytes = (uint32_t)(LW * LH + cc * SH * SW * 4);
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(bytes) : "memory");
-            const uint64_t tm0 = reinterpret_cast<uint64_t>(P.tmap_lat), tm1 = reinterpret_cast<uint64_t>(P.tmap_stk);
-            // the descriptors live in global memory (one pair per stream of the launch, written by the host)
-            if (P.use_tma & 2) {
-                asm volatile("fence.proxy.tensormap::generic.acquire.gpu [%0], 128;" ::"l"(tm0) : "memory");
-                asm volatile("fence.proxy.tensormap::generic.acquire.gpu [%0], 128;" ::"l"(tm1) : "memory");
-            }
-            asm volatile(
-                "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                ::"r"((uint32_t)__cvta_generic_to_shared(Lt)), "l"(tm0), "r"(lx0), "r"(ly0), "r"(bar_a)
-                : "memory");
-            asm volatile(
-                "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                ::"r"((uint32_t)__cvta_generic_to_shared(St)), "l"(tm1), "r"(sx0), "r"(sy0), "r"(0), "r"(bar_a)
-                : "memory");
-        }
-    } else {
-        for (int i = tid; i < LW * LH; i += SF_THREADS) {
-            const int r = i / LW, c = i - r * LW;
-            const int gy = ly0 + r, gx = lx0 + c;
-            Lt[i] = (gy >= 0 && gy < H && gx >= 0 && gx < W) ? P.lat[(size_t)gy * W + gx] : (int8_t)0;
-        }
-        for (int i = tid; i < cc * SH * SW; i += SF_THREADS) {
-            const int c = i / (SH * SW), rem = i - c * SH * SW, r = rem / SW, col = rem - r * SW;
-            const int gy = sy0 + r, gx = sx0 + col;
-            float v = 0.0f;
-            if (gy >= 0 && gy < ch && gx >= 0 && gx < cw)
-                v = P.stk8 ? (float)P.stk8[((size_t)c * ch + gy) * cw + gx] : __ldg(P.stk + ((size_t)c * ch + gy) * cw + gx);
-            St[i] = v;
-        }
-    }
-    // ---- weights (overlaps the bulk copies)
-    for (int i = tid; i < hid * CINP; i += SF_THREADS) {
-        const int hh = i / CINP, ci = i - hh * CINP;
-        sw0[i] = ci < cin ? P.w0[hh * cin + ci] : 0.0f;
-    }
-    for (int i = tid; i < hid; i += SF_THREADS) sb0[i] = P.b0[i];
-    for (int i = tid; i < hid * CP; i += SF_THREADS) {
-        const int hh = i / CP, c = i - hh * CP;
-        sw1[i] = c < C ? P.w1[c * hid + hh] : 0.0f;
-    }
-    for (int i = tid; i < CP; i += SF_THREADS) {
-        sb1[i] = i < C ? P.b1[i] : 0.0f;
-        sbs[i] = (i < C && P.stab_in) ? P.bs[i] : 0.0f;
-        sbo[i] = i < C ? P.bo[i] : 0.0f;
-        for (int l = 0; l < 2; l++) sb3[l * CP + i] = (i < C && l < n3) ? P.b3[l][i] : 0.0f;
-    }
-    for (int l = 0; l < n3; l++)
-        for (int i = tid; i < C * C * 9; i += SF_THREADS) sw3[l * C * C * 9 + i] = P.w3[l][i];
-    for (int i = tid; i < C * CINP; i += SF_THREADS) {
-        const int c = i / CINP, ci = i - c * CINP;
-        sws[i] = (ci < P.stab_in) ? P.ws[c * P.stab_in + ci] : 0.0f;
-    }
-    for (int i = tid; i < C * CP; i += SF_THREADS) {
-        const int c = i / CP, k = i - c * CP;
-        swo[i] = k < C ? P.wo[c * C + k] : 0.0f;
-    }
-    for (int i = tid; i < 64; i += SF_THREADS) skt[i] = P.kt[i >> 3][i & 7];
-    for (int i = tid; i < 49; i += SF_THREADS) skc[i] = P.kc[i / 7][i % 7];
-    if (P.use_tma) {
-        const uint32_t bar_a = (uint32_t)__cvta_generic_to_shared(bar);
-        uint32_t done = 0;
-        while (!done) {
-            asm volatile(
-                "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n selp.u32 %0, 1, 0, p;\n}\n"
-                : "=r"(done)
-                : "r"(bar_a)
-                : "memory");
-        }
-    }
-    __syncthreads();
-
-    // ---- stage A: last cascade level on the fly, then the two 1x1 layers (+ stabiliser on the tile itself), on the
-    // RH x RW region, 3 positions per thread
-    const int nA = RH * RW;
-    for (int base = 0; base < nA; base += 3 * SF_THREADS) {
-        float x[3][CINP], o[3][C];
-        int pos[3];
-#pragma unroll
-        for (int q = 0; q < 3; q++) {
-            const int pp = base + q * SF_THREADS + tid;
-            pos[q] = pp;
-            const int ppc = pp < nA ? pp : nA - 1;
-            const int py = ppc / RW, px = ppc - py * RW;
-            const int gy = clampi(Y0 + py, 0, H - 1), gx = clampi(X0 + px, 0, W - 1);
-#pragma unroll
-            for (int ci = 0; ci < CINP; ci++) x[q][ci] = 0.0f;
-            {
-                // channel 0: conv2d(latent, kron 7x7, zero padding) + latent   (upsampling.py:189-196)
-                const int8_t *lp = Lt + (gy - 3 - ly0) * LW + (gx - 3 - lx0);
-                float acc = 0.0f;
-#pragma unroll
-                for (int a = 0; a < 7; a++)
-#pragma unroll
-                    for (int b = 0; b < 7; b++) acc = __fmaf_rn(skc[a * 7 + b], (float)lp[a * LW + b], acc);
-                x[q][0] = __fadd_rn(acc, (float)lp[3 * LW + 3]);
-            }
-            {
-                // channels 1 .. cc: transposed conv (8x8 kron, stride 2, replicate-padded input, crop 11) of the
-                // coarser stack (upsampling.py:312-325): output (u, v) reads a 4 x 4 window, taps by parity
-                const int du = gy & 1, dv = gx & 1, qy = gy >> 1, qx = gx >> 1;
-                int ro[4], co[4];
-#pragma unroll
-                for (int t = 0; t < 4; t++) {
-                    ro[t] = (clampi(qy - 2 + du + t, 0, ch - 1) - sy0) * SW;
-                    co[t] = clampi(qx - 2 + dv + t, 0, cw - 1) - sx0;
-                }
-#pragma unroll
-                for (int c = 0; c < CINP - 1; c++) {
-                    if (c < cc) {
-                        const float *sp = St + c * SH * SW;
-                        float acc = 0.0f;
-#pragma unroll
-                        for (int t1 = 0; t1 < 4; t1++)
-#pragma unroll
-                            for (int t2 = 0; t2 < 4; t2++)
-                                acc = __fmaf_rn(skt[((1 - du) + 6 - 2 * t1) * 8 + (1 - dv) + 6 - 2 * t2], sp[ro[t1] + co[t2]], acc);
-                        x[q][c + 1] = acc;
-                    }
-                }
-            }
-#pragma unroll
-            for (int c = 0; c < C; c++) o[q][c] = sb1[c];
-        }
-        for (int hh = 0; hh < hid; hh++) {
-            float wv[CINP];
-#pragma unroll
-            for (int v = 0; v < CINP / 4; v++) {
-                const float4 t = *reinterpret_cast<const float4 *>(sw0 + hh * CINP + 4 * v);
-                wv[4 * v] = t.x; wv[4 * v + 1] = t.y; wv[4 * v + 2] = t.z; wv[4 * v + 3] = t.w;
-            }
-            float w1v[CP];
-#pragma unroll
-            for (int v = 0; v < CP / 4; v++) {
-                const float4 t = *reinterpret_cast<const float4 *>(sw1 + hh * CP + 4 * v);
-                w1v[4 * v] = t.x; w1v[4 * v + 1] = t.y; w1v[4 * v + 2] = t.z; w1v[4 * v + 3] = t.w;
-            }
-            const float bb = sb0[hh];
-#pragma unroll
-            for (int q = 0; q < 3; q++) {
-                float a = bb;
-#pragma unroll
-                for (int ci = 0; ci < CINP; ci++)
-                    if (ci < cin) a = __fmaf_rn(wv[ci], x[q][ci], a);
-                if (P.relu0) a = fmaxf(a, 0.0f);
-#pragma unroll
-                for (int c = 0; c < C; c++) o[q][c] = __fmaf_rn(w1v[c], a, o[q][c]);
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < 3; q++) {
-            if (pos[q] >= nA) continue;
-            const int py = pos[q] / RW, px = pos[q] - py * RW;
-#pragma unroll
-            for (int c = 0; c < C; c++) bufA[(c * RH + py) * RW + px] = P.relu1 ? fmaxf(o[q][c], 0.0f) : o[q][c];
-            const int ty = py - n3, tx = px - n3;
-            if (P.stab_in && ty >= 0 && ty < SF_TH && tx >= 0 && tx < SF_TW) {
-#pragma unroll
-                for (int c = 0; c < C; c++) {
-                    float a = sbs[c];
-#pragma unroll
-                    for (int ci = 0; ci < CINP; ci++)
-                        if (ci < P.stab_in) a = __fmaf_rn(sws[c * CINP + ci], x[q][ci], a);
-                    sstab[(c * SF_TH + ty) * SF_TW + tx] = a;
-                }
-            }
-        }
-    }
-    __syncthreads();
-    // ---- 3x3 layers, shared memory -> shared memory (the last one -> registers -> output)
-    const float *cur = bufA;
-    int cwid = RW, chh = RH, off = n3;
-    for (int l = 0; l < n3 - 1; l++) {
-        const int ow = cwid - 2, oh = chh - 2;
-        const float *wl = sw3 + l * C * C * 9;
-        for (int pp = tid; pp < ow * oh; pp += SF_THREADS) {
-            const int py = pp / ow, px = pp - py * ow;
-            const int gy = clampi(y0 - (off - 1) + py, 0, H - 1), gx = clampi(x0 - (off - 1) + px, 0, W - 1);
-            const int by = gy - (y0 - off), bx = gx - (x0 - off);
-            float acc[C];
-#pragma unroll
-            for (int co = 0; co < C; co++) acc[co] = sb3[l * CP + co];
-#pragma unroll
-            for (int ci = 0; ci < C; ci++)
-#pragma unroll
-                for (int ky = 0; ky < 3; ky++)
-#pragma unroll
-                    for (int kx = 0; kx < 3; kx++) {
-                        const float v = cur[(ci * chh + by + ky - 1) * cwid + bx + kx - 1];
-#pragma unroll
-                        for (int co = 0; co < C; co++) acc[co] = __fmaf_rn(wl[((co * C + ci) * 3 + ky) * 3 + kx], v, acc[co]);
-                    }
-#pragma unroll
-            for (int co = 0; co < C; co++) {
-                float a = acc[co];
-                if (P.res3[l]) a = __fadd_rn(a, cur[(co * chh + by) * cwid + bx]);
-                if (P.relu3[l]) a = fmaxf(a, 0.0f);
-                bufB[(co * oh + py) * ow + px] = a;
-            }
-        }
-        __syncthreads();
-        cur = bufB;
-        cwid = ow;
-        chh = oh;
-        off -= 1;
-    }
-    // ---- last stage on the tile: last 3x3 layer (if any), + stabiliser, output transform, frame tail, store
-    const size_t plane = (size_t)H * W;
-    const float M = P.M;
-    // 4:2:0 tail: rounded U, V samples of the tile [2][SF_TH][SF_TW], kept where the stabiliser output was (every
-    // thread has read its own position of it before it writes there)
-    float *uvq = sstab;
-    for (int pp = tid; pp < SF_TW * SF_TH; pp += SF_THREADS) {
-        const int ty = pp / SF_TW, tx = pp - ty * SF_TW;
-        const int gy = y0 + ty, gx = x0 + tx;
-        const bool inside = gy < H && gx < W;
-        const int by = (inside ? ty : 0) + off, bx = (inside ? tx : 0) + off;
-        float t[C];
-        if (n3 > 0) {
-            const int l = n3 - 1;
-            const float *wl = sw3 + l * C * C * 9;
-#pragma unroll
-            for (int co = 0; co < C; co++) t[co] = sb3[l * CP + co];
-#pragma unroll
-            for (int ci = 0; ci < C; ci++)
-#pragma unroll
-                for (int ky = 0; ky < 3; ky++)
-#pragma unroll
-                    for (int kx = 0; kx < 3; kx++) {
-                        const float v = cur[(ci * chh + by + ky - 1) * cwid + bx + kx - 1];
-#pragma unroll
-                        for (int co = 0; co < C; co++) t[co] = __fmaf_rn(wl[((co * C + ci) * 3 + ky) * 3 + kx], v, t[co]);
-                    }
-#pragma unroll
-            for (int co = 0; co < C; co++) {
-                if (P.res3[l]) t[co] = __fadd_rn(t[co], cur[(co * chh + by) * cwid + bx]);
-                if (P.relu3[l]) t[co] = fmaxf(t[co], 0.0f);
-            }
-        } else {
-#pragma unroll
-            for (int co = 0; co < C; co++) t[co] = cur[(co * chh + by) * cwid + bx];
-        }
-        if (P.stab_in) {
-#pragma unroll
-            for (int co = 0; co < C; co++) t[co] = __fadd_rn(t[co], sstab[(co * SF_TH + (inside ? ty : 0)) * SF_TW + (inside ? tx : 0)]);
-        }
-        float ov[C];
-#pragma unroll
-        for (int co = 0; co < C; co++) {
-            float a = sbo[co];
-#pragma unroll
-            for (int ci = 0; ci < C; ci++) a = __fmaf_rn(swo[co * CP + ci], t[ci], a);
-            ov[co] = a;
-        }
-        if (P.finish == 0) {
-            if (inside) {
-#pragma unroll
-                for (int co = 0; co < C; co++) P.out[co][(size_t)gy * W + gx] = ov[co];
-            }
-        } else if (P.finish == 1) {
-            if (inside) {
-#pragma unroll
-                for (int co = 0; co < C; co++) P.out[co][(size_t)gy * W + gx] = quant(clamp01(quant(ov[co], M)), M);
-            }
-        } else {
-            if (inside) P.out[0][(size_t)gy * W + gx] = quant(clamp01(quant(ov[0], M)), M);
-            uvq[(0 * SF_TH + ty) * SF_TW + tx] = quant(ov[1 < C ? 1 : 0], M);
-            uvq[(1 * SF_TH + ty) * SF_TW + tx] = quant(ov[2 < C ? 2 : 0], M);
-        }
-    }
-    (void)plane;
-    if (P.finish == 2) {
-        __syncthreads();
-        // 2 x 2 average of the rounded chroma samples in the order of the reference's avg_pool2d loop, clamp, round
-        const int h2 = H / 2, w2 = W / 2;
-        for (int pp = tid; pp < 2 * (SF_TW / 2) * (SF_TH / 2); pp += SF_THREADS) {
-            const int c = pp / ((SF_TW / 2) * (SF_TH / 2)), r = pp - c * (SF_TW / 2) * (SF_TH / 2);
-            const int by = r / (SF_TW / 2), bx = r - by * (SF_TW / 2);
-            const int y2 = y0 / 2 + by, x2 = x0 / 2 + bx;
-            if (y2 >= h2 || x2 >= w2) continue;
-            const float *q = uvq + (c * SF_TH + 2 * by) * SF_TW + 2 * bx;
-            float s = 0.0f;
-            s = __fadd_rn(s, q[0]);
-            s = __fadd_rn(s, q[1]);
-            s = __fadd_rn(s, q[SF_TW]);
-            s = __fadd_rn(s, q[SF_TW + 1]);
-            P.out[1 + c][(size_t)y2 * w2 + x2] = quant(clamp01(__fdiv_rn(s, 4.0f)), M);
-        }
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------------------
-// k_tail_syn2: same contract as k_tail_syn, restructured for instruction efficiency (k_tail_syn issues ~3 650
-// instructions per pixel for 862 FMAs):
+// k_tail_syn2, blocked for instruction efficiency (the first version of this kernel issued ~3 650 instructions per
+// pixel for 862 FMAs):
 //   * the halo of the stage-A region is rounded up to an even number of pixels, so that the region starts on even
 //     frame coordinates and stage A works on 2 x 2 QUADS with compile-time parities: the 8x8 stride-2 transposed
 //     conv reads ONE 5 x 5 window per channel for its four outputs, its taps come as 16 vector loads (re-laid
@@ -894,7 +557,7 @@ __global__ void __launch_bounds__(SF_THREADS) k_tail_syn(const TailSynJob *__res
 //     position's values (the 1x1 layers are pointwise), filled by a fix-up pass on border tiles only;
 //   * the 3x3 layers evaluate two horizontally adjacent outputs per thread from one 3 x 4 window per channel, their
 //     weights re-laid [ci][ky][kx][co] (one vector load per tap); stores are 64-bit.
-// Every output keeps its canonical accumulation order: bit-identical to k_tail_syn, k_syn_fused and the oracle.
+// Every output keeps its canonical accumulation order: bit-identical to k_syn_fused and the oracle.
 __host__ __device__ inline int ts2_n3e(int n3) { return (n3 + 1) & ~1; }
 constexpr int TS2_THREADS = 192;  // 180 quads per 32 x 16 tile with a 2-pixel halo; three CTAs per SM
 
@@ -1661,17 +1324,7 @@ PFN_encodeTiled get_encode_tiled() {
 }
 }  // namespace
 
-// development switch: CCD_TAIL_V=1 selects the first version of the fused tail kernel (k_tail_syn), default k_tail_syn2
-static int tail_version() {
-    static int v = 0;
-    if (!v) {
-        const char *e = getenv("CCD_TAIL_V");
-        v = (e && atoi(e) == 1) ? 1 : 2;
-    }
-    return v;
-}
-
-// Fills one TailSynJob (host memory).  Returns 1 when the tiles are staged with TMA, 0 when with plain loads
+// Fills one TailSynJob (host memory).  Returns 3 when the tiles are staged with TMA, 0 when with plain loads
 // (pitches / addresses that cuTensorMapEncodeTiled does not take), < 0 when the architecture is outside the family.
 int ccd_tail_fill_syn(void *dst, const CcdTailSynDesc &T) {
     const int n_layers = T.n_layers;
@@ -1721,7 +1374,7 @@ int ccd_tail_fill_syn(void *dst, const CcdTailSynDesc &T) {
         (reinterpret_cast<uintptr_t>(T.stk) % 16) == 0) {
         const uint64_t gd0[2] = {(uint64_t)T.w, (uint64_t)T.h};
         const uint64_t gs0[1] = {(uint64_t)T.w};
-        const int n3t = tail_version() == 2 ? ts2_n3e(J.n3) : J.n3;  // halo of the staged tiles
+        const int n3t = ts2_n3e(J.n3);  // halo of the staged tiles
         const uint32_t bx0[2] = {(uint32_t)ts_lw(n3t), (uint32_t)ts_lh(n3t)};
         const uint32_t es[3] = {1, 1, 1};
         const uint64_t gd1[3] = {(uint64_t)T.cw, (uint64_t)T.ch, (uint64_t)cc};
@@ -1730,10 +1383,6 @@ int ccd_tail_fill_syn(void *dst, const CcdTailSynDesc &T) {
         const int r0 = enc(J.tmap_lat, 0, 2, const_cast<int8_t *>(T.lat), gd0, gs0, bx0, es, 0, 0, 1, 0);
         const int r1 = enc(J.tmap_stk, 7, 3, const_cast<float *>(T.stk), gd1, gs1, bx1, es, 0, 0, 1, 0);
         J.use_tma = (r0 == 0 && r1 == 0) ? 3 : 0;  // bit 0: TMA staging, bit 1: descriptor fence before the first use
-        if (J.use_tma) {
-            const char *e = getenv("CCD_TMA_MODE");  // development switch: 0 plain loads, 1 TMA, 3 TMA + descriptor fence
-            if (e) J.use_tma = atoi(e);
-        }
     }
     memcpy(dst, &J, sizeof(J));
     return J.use_tma;
@@ -1742,26 +1391,21 @@ int ccd_tail_fill_syn(void *dst, const CcdTailSynDesc &T) {
 template <int CINP, int C>
 static int launch_tail_syn(const void *d_jobs, int n_jobs, int n3_max, int hid_max, int max_w, int max_h, cudaStream_t st) {
     constexpr int CP = (C + 3) & ~3;
-    const bool v2 = tail_version() == 2;
-    const int n3t = v2 ? ts2_n3e(n3_max) : n3_max;
+    const int n3t = ts2_n3e(n3_max);
     const int RW = SF_TW + 2 * n3t, RH = SF_TH + 2 * n3t;
     size_t bytes = 128 + (((size_t)ts_lw(n3t) * ts_lh(n3t) + 127) & ~(size_t)127);
     size_t fl = (((size_t)(CINP - 1) * ts_sh(n3t) * ts_sw(n3t) + 31) & ~(size_t)31);
-    if (v2) {
-        fl += (size_t)ts_lw(n3t) * ts_lh(n3t);
-        fl += (size_t)hid_max * CINP + ((hid_max + 3) & ~3) + (size_t)hid_max * CP + CP + 2 * C * 9 * CP + 2 * CP + C * CINP + CP + C * CP + CP + 64 + 56;
-    } else {
-        fl += (size_t)hid_max * CINP + hid_max + (size_t)hid_max * CP + CP + 2 * C * C * 9 + 2 * CP + C * CINP + CP + C * CP + CP + 64 + 52;
-    }
+    fl += (size_t)ts_lw(n3t) * ts_lh(n3t);
+    fl += (size_t)hid_max * CINP + ((hid_max + 3) & ~3) + (size_t)hid_max * CP + CP + 2 * C * 9 * CP + 2 * CP + C * CINP + CP + C * CP + CP + 64 + 56;
     fl += (size_t)C * RH * RW + (n3_max == 2 ? (size_t)C * (RH - 2) * (RW - 2) : 0) + (size_t)C * SF_TH * SF_TW;
     const size_t smem = bytes + fl * sizeof(float);
-    auto kern = v2 ? k_tail_syn2<CINP, C> : k_tail_syn<CINP, C>;
+    auto kern = k_tail_syn2<CINP, C>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
     }
     const dim3 grid((max_w + SF_TW - 1) / SF_TW, (max_h + SF_TH - 1) / SF_TH, (unsigned)n_jobs);
-    kern<<<grid, v2 ? TS2_THREADS : SF_THREADS, smem, st>>>(reinterpret_cast<const TailSynJob *>(d_jobs));
+    kern<<<grid, TS2_THREADS, smem, st>>>(reinterpret_cast<const TailSynJob *>(d_jobs));
     g_ccd_launches++;
     return (int)cudaGetLastError();
 }

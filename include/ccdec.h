@@ -242,10 +242,6 @@ int ccd_debug_laplace_domain(CcdContext *ctx, int sc_lo, int sc_hi, uint32_t *ou
 /* Number of CUDA kernels this library has launched since it was loaded. */
 uint64_t ccd_debug_launch_count(void);
 
-/* Tuning knob: which of warps 0..14 of the entropy CTA act as ARM producers (bit i = warp i;
- * warp 14 is the coder's helper, warp 15 the range coder).  Default 0x3777: warps 3, 7, 11 stay idle so
- * that the coder owns scheduler partition 3. */
-int ccd_debug_set_producer_mask(CcdContext *ctx, uint32_t mask);
 /* 1 (default): one fused kernel for the synthesis when the architecture allows it; 0: one kernel per
  * layer.  Both give bit-identical results (tests/test_gpu_decode.py). */
 int ccd_debug_set_fused_synthesis(CcdContext *ctx, int on);

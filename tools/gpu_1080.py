@@ -9,8 +9,6 @@ from coolchic_b200._desc import desc_from_header
 ctx = _native.get_context(0)
 ss = synth.SeedStream(ctx)
 hyp = (4, 6) if "hyper" in sys.argv else None
-for a_ in sys.argv[1:]:
-    if a_.startswith("mask="): ctx._lib.ccd_debug_set_producer_mask(ctx._h, int(a_[5:], 0))
 zeros = "zeros" in sys.argv
 lat_in = None
 if zeros:  # all-zero latents: (almost) every symbol is the mode -> time per symbol = the coder's hot path

@@ -12,7 +12,6 @@ v = VideoHeader(); rest = v.read_header(data); f = FrameHeader(); rest = f.read_
 d = desc_from_header(c)
 nnb = rest[:c.get_value("nn_n_bytes")]; lb = rest[c.get_value("nn_n_bytes"):][:c.get_value("n_bytes_latent")]
 ctx = _native.get_context(0)
-if len(sys.argv) > 2: ctx._lib.ccd_debug_set_producer_mask(ctx._h, int(sys.argv[2], 0))
 nn = _native.decode_nn(d, nnb)
 g = np.load(os.path.join(ROOT, "tests/golden/kodim14_latents.npz"))["latents"]
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 20
